@@ -2,7 +2,7 @@
 """bench.py - image-pairs/sec on synthetic pairs (BASELINE.json configs 2-5; default config 2 = 480x640).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2|3|4|5]
-                    [--engine f16x3|fp32|f16|tf32] [--lanes L] [--pairs-per-step P]
+                    [--engine f16x3|fp32|f16|tf32] [--lanes L] [--pairs-per-step P] [--dump-outputs DIR]
 
 One "step" = P independent pairs per GPU (default 32, `config.pairs_per_gpu_per_step`), each through the whole hot path
 (variant-A CoarseAlign.setPair -> getCoarse -> warp_grid -> PredFlowMask).  Config 2: nbScale 7, scaleR 2, nbIter 1000, one
@@ -217,6 +217,49 @@ def states():
             synth.net_matchability_state(2))
 
 
+DUMP_SAMPLE = 1 << 16          # elements kept of a larger output array (a seeded sample): a step's dump stays far below 64 MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _dump_leaves(name, v):
+    """(name, value) for every array-like leaf of a result: dict keys and list positions join the name with '_'."""
+    if isinstance(v, dict):
+        for k, x in v.items():
+            yield from _dump_leaves("%s_%s" % (name, k), x)
+    elif isinstance(v, (list, tuple)) and not all(isinstance(x, (int, float, np.number)) for x in v):
+        for j, x in enumerate(v):
+            yield from _dump_leaves("%s_%d" % (name, j), x)
+    else:
+        yield name, v
+
+
+def dump_outputs(outs, d):
+    """Write the per-pair results of one step as d/pair<r>_<key>.npy: integers and float64 data as float64, the rest as float32;
+    an array of more than DUMP_SAMPLE elements as the same seeded sample of its flat elements in every run.  A CUDA tensor is
+    written only for the last result that holds its storage: the graphed aligners return flow12 as the graph's output buffer
+    (copy=False), which the lane's next pair overwrites."""
+    import torch
+    leaves = [leaf for r, out in enumerate(outs) for leaf in _dump_leaves("pair%02d" % r, out)]
+    owner = {v.data_ptr(): name for name, v in leaves if isinstance(v, torch.Tensor) and v.is_cuda}
+    arrays = {}
+    for name, v in leaves:
+        if isinstance(v, torch.Tensor):
+            if v.is_cuda and owner[v.data_ptr()] != name:
+                continue
+            v = v.detach().cpu().numpy()
+        a = np.asarray(v)
+        a = a.astype(np.float64 if a.dtype.kind in "iu" or a.dtype == np.float64 else np.float32)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.RandomState(a.size).choice(a.size, DUMP_SAMPLE, replace=False))]
+        arrays[name] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %.1f MB (limit %d MB); use fewer --pairs-per-step" % (total / 1e6, DUMP_MAX_BYTES >> 20))
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- reference arm (CPU oracle)
 def run_reference(args, rank, world):
     """The reference's own algorithm on the host cores (oracle/pair_oracle.py, torch-CPU fp32).  With --dump-parity FILE it
@@ -423,6 +466,11 @@ def run_b200(args, rank, world, local):
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
+        # the graphs draw their RANSAC samples from CUDA generator states whose offsets the time-bounded pre-warm leaves wherever
+        # it stopped: reseeding makes the timed steps see the same samples in every run
+        torch.cuda.manual_seed(1000)
+        if multi is not None:
+            multi.manual_seed(1000)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = rf._lib.launch_count() + replayed()
         e0.record()
@@ -452,7 +500,7 @@ def run_b200(args, rank, world, local):
             tmax = torch.tensor([ms], device=dev)
             dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
             ms = float(tmax.item())
-        return ms, launches, outs[-1], allr, gather_ms
+        return ms, launches, outs, allr, gather_ms
 
     # set-up, untimed and before the W warm-up steps of the contract: a couple of seconds of the real load (clocks, power state,
     # allocator).  Observation (profiles/README.md): with device-resident inputs every other 32-pair step takes ~139 instead of
@@ -471,8 +519,12 @@ def run_b200(args, rank, world, local):
             step(i_pre, False)
             i_pre += 1
         torch.cuda.synchronize()
-    ms_dev, launches, out, _, _ = timed(False, args.steps, args.warmup)
-    ms_e2e, _, out, allr, gather_ms = timed(True, args.steps, max(1, args.warmup // 2))
+    ms_dev, launches, outs, _, _ = timed(False, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(outs, args.dump_outputs)                     # before the next region's replays overwrite the graphs' buffers
+    del outs                                                      # the e2e region allocates its results in the memory these held
+    ms_e2e, _, outs, allr, gather_ms = timed(True, args.steps, max(1, args.warmup // 2))
+    out = outs[-1]
     clocks = sampler.stop() if rank == 0 else None
     assert allr.shape[0] == args.steps * P * world
     if os.environ.get("RF_BENCH_REPEAT_RESIDENT") and rank == 0 and world == 1:      # experiment: order dependence of the two timed regions
@@ -641,6 +693,8 @@ def main():
                     help="pairs per GPU and step (default 32 for configs 2 / 3, 8 for config 4, 4 for config 5)")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="launch the kernels of a pair one by one instead of replaying a CUDA graph")
     ap.add_argument("--dump-parity", default=None, help="(reference arm) write the oracle's outputs for pair 0 to this .npz")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the results of the last timed step (the region `value` times) to DIR/<name>.npy; same arguments, same inputs")
     args = ap.parse_args()
     if args.pairs_per_step <= 0:
         args.pairs_per_step = {2: 32, 3: 32, 4: 8, 5: 4}[args.config]

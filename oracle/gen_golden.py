@@ -29,6 +29,8 @@ from . import warp_oracle as WO
 
 REF = os.environ.get("RF_REFERENCE", "/root/reference")
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# torch-CPU threads the golden outputs are computed with: the reduction order of the convolutions depends on it
+GOLDEN_THREADS = 8
 
 
 def _load(name, path):
@@ -466,9 +468,52 @@ def gen_metrics():
          XA=XA, YA=YA, XB=XB, YB=YB, pixelGrid=pixelGrid, dims=np.array([wB, hB, wA, hA]), counts=np.asarray(cnt), nbAlign=np.int64(nb))
 
 
+DROPIN_SCRIPTS = ["quick_start/align2images.py", "evaluation/evalHpatch/evaluation.py", "evaluation/evalCorr/evaluation.py",
+                  "evaluation/evalKITTI/evaluation.py", "evaluation/evalYFCC/evaluation.py", "evaluation/evalHpatch/getResults.py",
+                  "evaluation/evalCorr/getResults.py", "evaluation/evalKITTI/getResults.py"]
+
+
+def script_uses(path):
+    """What one driver script uses of the drop-in modules, read from its AST: attributes of ``outil`` / ``model`` / ``tgm``,
+    the positional count and keyword names of every ``CoarseAlign(...)`` assignment, the attributes read on names bound to a
+    CoarseAlign instance, and the names imported from ``coarseAlignFeatMatch``."""
+    tree = ast.parse(open(path).read())
+    mod_attrs, ctor_calls, inst_attrs, imports = set(), [], set(), set()
+    inst_names = set()
+    for node in ast.walk(tree):
+        if isinstance(node, ast.Assign) and isinstance(node.value, ast.Call) and isinstance(node.value.func, ast.Name) \
+                and node.value.func.id == "CoarseAlign":
+            ctor_calls.append({"nargs": len(node.value.args), "keywords": [k.arg for k in node.value.keywords if k.arg]})
+            for t in node.targets:
+                if isinstance(t, ast.Name):
+                    inst_names.add(t.id)
+        if isinstance(node, ast.ImportFrom) and node.module == "coarseAlignFeatMatch":
+            imports.update(al.name for al in node.names)
+    for node in ast.walk(tree):
+        if isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name):
+            if node.value.id in ("outil", "model", "tgm"):
+                mod_attrs.add(node.value.id + "." + node.attr)
+            if node.value.id in inst_names:
+                inst_attrs.add(node.attr)
+    return {"module_attrs": sorted(mod_attrs), "coarse_align_calls": ctor_calls,
+            "coarse_align_attrs": sorted(inst_attrs), "coarse_align_imports": sorted(imports)}
+
+
+def gen_script_uses():
+    """tests/golden/dropin_script_uses.json: the drop-in API surface each of the reference's driver scripts relies on."""
+    import json
+    os.makedirs(OUT, exist_ok=True)
+    uses = {s: script_uses(os.path.join(REF, s)) for s in DROPIN_SCRIPTS}
+    with open(os.path.join(OUT, "dropin_script_uses.json"), "w") as f:
+        json.dump(uses, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("wrote dropin_script_uses", {s: len(u["module_attrs"]) for s, u in uses.items()})
+
+
 def main():
     assert os.path.isdir(REF), "reference checkout not found at %s" % REF
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_THREADS)
+    gen_script_uses()
     gen_outil()
     gen_models()
     gen_pred_flow_mask()

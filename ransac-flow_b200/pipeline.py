@@ -190,6 +190,7 @@ class GraphedAligner:
         self.graphs = {}                # insertion-ordered: least recently used first
         self.max_graphs = max_graphs    # datasets with many image sizes (HPatches, MegaDepth, YFCC): LRU-bounded graph memory
         self.replayed_kernels = 0       # library kernels executed through graph replays (they bypass rf_launch_count)
+        self.rng = None                 # generator state the graphs draw their samples from (None: the default CUDA generator's)
 
     def _device(self, s_in, t_in):
         """The device work of one pair, queued on the current stream: (packed results, flow12 | None, (H, W), flowDown8 shape)."""
@@ -220,6 +221,18 @@ class GraphedAligner:
         del rec
 
     def _build(self, Is, It):
+        if self.rng is None:
+            return self._capture(Is, It)
+        d = torch.cuda.current_device()
+        gen = torch.cuda.default_generators[d]
+        default_state = gen.graphsafe_get_state()
+        gen.graphsafe_set_state(self.rng)            # the graph registers (and its replays advance) this state, not the default
+        try:
+            return self._capture(Is, It)
+        finally:
+            gen.graphsafe_set_state(default_state)
+
+    def _capture(self, Is, It):
         dev = torch.device("cuda", torch.cuda.current_device())
         s_in = torch.empty(tuple(Is.shape), dtype=torch.uint8, device=dev)
         t_in = torch.empty(tuple(It.shape), dtype=torch.uint8, device=dev)
@@ -389,6 +402,18 @@ class ConcurrentAligner:
         mk = make_aligner or (lambda c, n: GraphedAligner(c, n, with_match21=with_match21))
         self.lanes = [mk(*make_models()) for _ in range(lanes)]
         self.streams = [torch.cuda.Stream() for _ in range(lanes)]
+        # a replay writes its generator state's seed / offset into device tensors on its own stream: lanes replayed side by
+        # side must not share a state, or a lane's RANSAC draws with whichever offset another lane wrote last
+        d = torch.cuda.current_device()
+        default = torch.cuda.default_generators[d]
+        for a in self.lanes:
+            a.rng = default.clone_state()
+        self.manual_seed(default.initial_seed())
+
+    def manual_seed(self, seed):
+        """Seed lane k's generator with ``seed + k`` (distinct sample streams; ``torch.manual_seed`` does not reach them)."""
+        for k, a in enumerate(self.lanes):
+            a.rng.manual_seed(seed + k)
 
     @property
     def replayed_kernels(self):

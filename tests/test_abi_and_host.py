@@ -187,6 +187,34 @@ def test_bench_roofline_record_is_complete():
     assert abs(bench.roofline_record(1, False, 0.24, 0.04, 10, pk)["executed_tensor_frac"] - 6 * (32.108544 / 0.24) / 1703.4) < 1e-9
 
 
+def test_bench_dump_outputs_names_dtypes_and_sample(tmp_path):
+    """bench.py --dump-outputs: one float .npy per result leaf, large arrays as the same seeded sample every time, and no dump
+    over 64 MB."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rs = np.random.RandomState(0)
+    big = rs.rand(480, 640).astype(np.float32)
+    outs = [dict(H=rs.rand(1, 3, 3), flowDown8=rs.rand(1, 2, 60, 80).astype(np.float32), match=[big], nbInlier=17, size=(480, 640),
+                 maps=[(big > 0.5, np.arange(3))]) for _ in range(2)]
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(outs, str(d))
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted("pair%02d_%s.npy" % (r, k) for r in range(2)
+                           for k in ("H", "flowDown8", "match_0", "nbInlier", "size", "maps_0_0", "maps_0_1"))
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), n
+    assert np.array_equal(np.load(tmp_path / "a" / "pair00_H.npy"), outs[0]["H"])
+    assert np.load(tmp_path / "a" / "pair01_nbInlier.npy") == 17 and np.load(tmp_path / "a" / "pair00_size.npy").dtype == np.float64
+    m = np.load(tmp_path / "a" / "pair00_match_0.npy")
+    assert m.shape == (bench.DUMP_SAMPLE,) and np.isin(m, big).all()
+    with pytest.raises(SystemExit):
+        bench.dump_outputs([dict(match=[big])] * (bench.DUMP_MAX_BYTES // (4 * bench.DUMP_SAMPLE) + 1), str(tmp_path / "c"))
+    assert not (tmp_path / "c").exists()
+
+
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU oracle timed on the host cores; rank 0 only under torchrun) prints ONE JSON line with
     the contract's keys; a non-zero rank prints nothing and exits 0."""

@@ -1,75 +1,52 @@
 """The drop-in boundary against the reference's REAL driver scripts (SURVEY 8b).
 
-CPU part (runs where the reference checkout exists, i.e. in the build container; skipped elsewhere): every driver script is
-parsed and each use it makes of the drop-in modules - names imported from them, constructor calls and their argument
-counts / keywords, methods and attributes read on the CoarseAlign object, on the networks and on the warper - is checked
-against this package's mirrors.  A script cannot run end to end here (no GPU in the build container; the reference
-checkout does not exist on the GPU box), so the GPU part re-enacts the statement sequence of quick_start/align2images.py in
-a driver of its own, run byte-for-byte through ``dropin.main`` with torch's own F.grid_sample / F.interpolate between the
-calls exactly as the script mixes them, and compares what it saves with the CPU oracle."""
-import ast
+CPU part: each use a driver script makes of the drop-in modules - names imported from them, constructor calls and their
+argument counts / keywords, methods and attributes read on the CoarseAlign object, on the networks and on the warper - is
+checked against this package's mirrors.  Those uses were read from the scripts' ASTs by ``oracle/gen_golden.py``
+(``gen_script_uses``) and are stored in tests/golden/dropin_script_uses.json, so the check needs no reference checkout.
+The GPU part re-enacts the statement sequence of quick_start/align2images.py in a driver of its own, run byte-for-byte
+through ``dropin.main`` with torch's own F.grid_sample / F.interpolate between the calls exactly as the script mixes them,
+and compares what it saves with the CPU oracle."""
 import inspect
+import json
 import os
 import sys
 
 import numpy as np
 import pytest
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+with open(os.path.join(GOLDEN, "dropin_script_uses.json")) as _f:
+    SCRIPT_USES = json.load(_f)
 SCRIPTS = ["quick_start/align2images.py", "evaluation/evalHpatch/evaluation.py", "evaluation/evalCorr/evaluation.py",
            "evaluation/evalKITTI/evaluation.py", "evaluation/evalYFCC/evaluation.py", "evaluation/evalHpatch/getResults.py",
            "evaluation/evalCorr/getResults.py", "evaluation/evalKITTI/getResults.py"]
 
 
-def _uses(tree):
-    """(module attribute uses, CoarseAlign call nodes, names bound to a CoarseAlign instance -> attributes read on them)."""
-    mod_attrs, ctor_calls, inst_attrs = set(), [], {}
-    inst_names = set()
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Assign) and isinstance(node.value, ast.Call) and isinstance(node.value.func, ast.Name) \
-                and node.value.func.id == "CoarseAlign":
-            ctor_calls.append(node.value)
-            for t in node.targets:
-                if isinstance(t, ast.Name):
-                    inst_names.add(t.id)
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name):
-            if node.value.id in ("outil", "model", "tgm"):
-                mod_attrs.add((node.value.id, node.attr))
-            if node.value.id in inst_names:
-                inst_attrs.setdefault(node.value.id, set()).add(node.attr)
-    return mod_attrs, ctor_calls, inst_attrs
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout is only present in the build container")
 @pytest.mark.parametrize("script", SCRIPTS)
 def test_reference_script_api_surface_is_covered(rf, script):
     from ransac_flow_b200 import dropin
-    path = os.path.join(REF, script)
-    tree = ast.parse(open(path).read())
-    variant = dropin.variant_for(path)
+    uses = SCRIPT_USES[script]
+    variant = dropin.variant_for(os.path.join(os.sep, script))
     cls = {"A": rf.CoarseAlignA, "B": rf.CoarseAlignB, "C": rf.CoarseAlignC}[variant]
-    mod_attrs, ctor_calls, inst_attrs = _uses(tree)
     mirrors = {"outil": rf.outil, "model": rf.model, "tgm": rf.kornia_geometry}
-    for m, a in sorted(mod_attrs):
-        assert hasattr(mirrors[m], a), "%s uses %s.%s, which the mirror lacks" % (script, m, a)
+    for use in uses["module_attrs"]:
+        m, a = use.split(".")
+        assert hasattr(mirrors[m], a), "%s uses %s, which the mirror lacks" % (script, use)
     sig = inspect.signature(cls.__init__)
-    for call in ctor_calls:                                    # the script's own positional count and keyword names must bind
-        args = [None] * (1 + len(call.args))
-        kwargs = {k.arg: None for k in call.keywords if k.arg}
+    for call in uses["coarse_align_calls"]:                    # the script's own positional count and keyword names must bind
+        args = [None] * (1 + call["nargs"])
+        kwargs = {k: None for k in call["keywords"]}
         sig.bind(*args, **kwargs)
-    for name, attrs in inst_attrs.items():
-        for a in attrs:
-            assert hasattr(cls, a) or a in ("Is", "It", "IsTensor", "ItTensor", "featt", "scaleList", "Wt", "Ht", "featsMultiScale"), \
-                "%s reads CoarseAlign.%s" % (script, a)
+    for a in uses["coarse_align_attrs"]:
+        assert hasattr(cls, a) or a in ("Is", "It", "IsTensor", "ItTensor", "featt", "scaleList", "Wt", "Ht", "featsMultiScale"), \
+            "%s reads CoarseAlign.%s" % (script, a)
     # the bare module names the script imports resolve after install()
     saved = {k: sys.modules.get(k) for k in ("coarseAlignFeatMatch", "outil", "model", "kornia", "kornia.geometry")}
     try:
         dropin.install(variant)
-        for node in ast.walk(tree):
-            if isinstance(node, ast.ImportFrom) and node.module == "coarseAlignFeatMatch":
-                for al in node.names:
-                    assert hasattr(sys.modules["coarseAlignFeatMatch"], al.name)
+        for name in uses["coarse_align_imports"]:
+            assert hasattr(sys.modules["coarseAlignFeatMatch"], name)
     finally:
         for k, v in saved.items():
             if v is None:

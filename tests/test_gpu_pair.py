@@ -337,6 +337,31 @@ def test_concurrent_aligner_equals_graphed_aligner(rf):
         rf.outil.corr_precision = 0
 
 
+def test_concurrent_aligner_lanes_are_reproducible_after_manual_seed(rf):
+    """Each lane's graphs draw their RANSAC samples from the lane's own generator state, so lanes released together do not
+    race on one generator's offset: after ConcurrentAligner.manual_seed the same pairs give bit-identical results."""
+    rf.model.set_engine("f16")
+    rf.outil.corr_precision = 2
+    try:
+        rsd = synth.resnet50_conv4_state(0)
+
+        def make_models():
+            c = rf.CoarseAlignA(3, 1000, 0.05, "Homography", 96, 2, False, 2, True, False, resnet_state_dict=rsd, verbose=False)
+            return c, networks(rf)
+        pairs = [tuple(torch.from_numpy(a).cuda() for a in synth.make_pair(40 + i, 96, 128)[:2]) for i in range(4)]
+        multi = rf.pipeline.ConcurrentAligner(make_models, lanes=4)
+        multi.prepare(*pairs[0])
+        runs = []
+        for _ in range(2):
+            multi.manual_seed(3)
+            runs.append(multi.run(pairs * 3))
+        for a, b in zip(*runs):
+            assert np.array_equal(a["H"], b["H"]) and a["nbInlier"] == b["nbInlier"] and np.array_equal(a["flowDown8"], b["flowDown8"])
+    finally:
+        rf.model.set_engine("fp32")
+        rf.outil.corr_precision = 0
+
+
 def test_graphed_aligner_results_survive_later_replays_and_graph_eviction(rf):
     """ADVICE r1: (1) a result kept across replays must not be overwritten (flow12 used to alias the graph's static buffer);
     (2) graphs are LRU-bounded and an evicted graph takes the activation buffers only it used with it - replaying the
