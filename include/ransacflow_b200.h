@@ -55,11 +55,10 @@ uint64_t rf_launch_count(void);
  * precision: 0 = exact fp32 FMA (SIMT); 1 = 3xTF32 on tcgen05 tensor cores (hi*hi + lo*hi + hi*lo, C % 32 == 0);
  * 2 = fp16 split on tcgen05 (x = hi + lo * 2^-11 in fp16, cross terms in a second TMEM accumulator, C % 64 == 0): the
  * same 22 significand bits with half the MMAs per channel.
- * Precision 2 has two kernel sequences with identical outputs (environment RF_CORR_V2, read per call): the persistent
- * correlation kernel (one CTA per SM, two TMEM accumulator pairs, arg-max epilogue overlapped with the next tile's
- * MMAs) between a fused split / key-zeroing launch and a fused mutual-test + compaction launch (3 launches), or the
- * one-tile-per-CTA kernel with separate helpers (6 launches).  rf_corr_mutual_nn_launches() (host only) tells which
- * one a call with this precision would run now: it returns the number of launches. */
+ * Precision 2 runs the persistent correlation kernel (one CTA per SM, two TMEM accumulator pairs, arg-max epilogue
+ * overlapped with the next tile's MMAs) between a fused split / key-zeroing launch and a fused mutual-test + compaction
+ * launch.  rf_corr_mutual_nn_launches() (host only) returns the number of launches a call with this precision makes
+ * (NA, NB > 0): 4 / 6 / 3 for precision 0 / 1 / 2. */
 size_t rf_corr_mutual_nn_workspace(int NA, int NB, int C, int precision);
 int rf_corr_mutual_nn_launches(int precision);
 int rf_corr_mutual_nn(const float* featA, int NA, const float* featB, int NB, int C,

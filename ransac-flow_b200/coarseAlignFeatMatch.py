@@ -86,7 +86,7 @@ class ResNet50Conv4:
         if eng == ops.ENGINE_SPLIT:
             if self._program_split is None:
                 # the fp16 program's topology with the weights read as hi / lo planes; conv3 + down-sampling branch fused
-                self._program_split = self._build(64, fuse_downsample=os.environ.get("RF_FUSE_DOWNSAMPLE", "1") != "0")
+                self._program_split = self._build(64, fuse_downsample=True)
             out, ohw = self._program_split.run(x, eng)
         elif eng == ops.ENGINE_F16:
             if self._program_f16 is None:
@@ -174,7 +174,7 @@ class _CoarseAlignBase:
         flat = torch.cat([t.reshape(-1, 3) for t in u8], dim=0) if len(u8) > 1 else u8[0].reshape(-1, 3)
         x = Ragged(ops.preproc_u8(flat, normalize=True), hw)
         f = self.net(x)
-        if f.split and outil.corr_precision == 2 and os.environ.get("RF_CORR_PRESPLIT", "1") != "0":
+        if f.split and outil.corr_precision == 2:
             # engine 'f16x3' + fp16-split correlation: the normalisation writes the correlation's operand planes directly;
             # the fp32 views the reference exposes (featsMultiScale, featt) are rebuilt on first access (__getattr__)
             return Ragged(ops.l2norm_planes(f.data), f.hw), u8
@@ -279,9 +279,7 @@ class CoarseAlignA(_CoarseAlignBase):
                  segNet=True, resnet_state_dict=None, verbose=True):
         self._setup(nbScale, nbIter, tolerance, transform, minSize, scaleR, imageNet, segNet, resnet_state_dict, verbose)
 
-    def setPair(self, Is_org, It_org, after_preproc=None):
-        """``after_preproc`` (optional callable): invoked as soon as ``ItTensor`` / ``IsTensor`` exist, before the ResNet
-        trunk is queued - the pair pipeline uses it to start the target's fine features on a second stream."""
+    def setPair(self, Is_org, It_org):
         with torch.no_grad():
             ws, hs = self._size_of(Is_org)
             sizes = [self._target_size(ws, hs, int(self.minSize * s)) for s in self.scaleList]
@@ -295,8 +293,6 @@ class CoarseAlignA(_CoarseAlignBase):
             self.Is, self.It = self._as_pil(IsList[mid]), self._as_pil(ItR)
             self.IsTensor = self._to_tensor01(u8[mid])
             self.ItTensor = self._to_tensor01(u8[nS])
-            if after_preproc is not None:
-                after_preproc()
             feats, _ = self._features(u8)                         # 7 scales + target: one ragged batch
             self._set_source_feats(feats, nS)
             self._set_target_feats(feats, nS)

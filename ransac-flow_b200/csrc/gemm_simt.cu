@@ -11,7 +11,6 @@
 // (transposed on the store so fragment reads are 128-bit and conflict free),
 // global loads of slice k+1 in flight while slice k is multiplied.
 // The tcgen05 tensor-core engine (gemm_tc.cu) replaces these where TF32 is allowed.
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -310,8 +309,7 @@ mutual_cols_compact_kernel(const unsigned long long* __restrict__ rowbest, const
 static int launch_mutual_compact(const unsigned long long* rowbest, const unsigned long long* colbest, int NA, int NB, long long* idx1, long long* idx2,
                                  int* count, cudaStream_t st) {
     const size_t smem = (size_t)NA * sizeof(int);
-    const char* e = getenv("RF_COMPACT_COLS");                    // 1 (default): column-driven compaction; 0: the row-driven kernel
-    if ((e ? atoi(e) : 1) && smem <= 200 * 1024) {
+    if (smem <= 200 * 1024) {                                      // the row table fits in shared memory: column-driven compaction
         static bool attr[64] = {false};
         const int dev = current_device();
         if (!attr[dev]) {
@@ -513,9 +511,8 @@ using namespace rf;
 
 // tensor-core engines live in gemm_tc.cu
 int rf_corr_argmax_tc(const float* featA, int NA, const float* featB, int NB, int C,
-                      unsigned long long* rowbest, unsigned long long* colbest, void* ws, cudaStream_t st, int precision, bool v2,
-                      const void* const* presplit = nullptr, void* const* tail = nullptr);
-int rf_corr_v2_mode();
+                      unsigned long long* rowbest, unsigned long long* colbest, void* ws, cudaStream_t st, int precision,
+                      const void* const* presplit = nullptr);
 size_t rf_corr_tc_workspace(int NA, int NB, int C);
 int rf_conv2d_tc(const ImgSet& set, const ConvParams& p, const void* w_tc, cudaStream_t st, bool f16, bool out32);
 bool rf_conv2d_tc_supported(const ConvParams& p);
@@ -532,7 +529,7 @@ extern "C" size_t rf_corr_mutual_nn_workspace(int NA, int NB, int C, int precisi
 }
 
 extern "C" int rf_corr_mutual_nn_launches(int precision) {
-    if (precision == 2 && rf_corr_v2_mode() != 0) return 3;          // split+zero, persistent correlation, flag+compact
+    if (precision == 2) return 3;                                    // split+zero, persistent correlation, flag+compact
     return precision == 0 ? 4 : 6;                                   // memset, [split, split,] correlation, flag, compact
 }
 
@@ -545,14 +542,14 @@ extern "C" int rf_corr_mutual_nn(const float* featA, int NA, const float* featB,
     cudaStream_t st = as_stream(stream);
     unsigned long long* rowbest = reinterpret_cast<unsigned long long*>(ws);
     unsigned long long* colbest = rowbest + NA;
-    // precision 2 with RF_CORR_V2: persistent correlation kernel; its split launch zeroes the keys, and the mutual test
-    // and the compaction are one kernel (3 launches instead of 6)
-    const bool v2 = precision == 2 && NA > 0 && NB > 0 && rf_corr_v2_mode() != 0;
-    if (!v2) RF_CUDA(cudaMemsetAsync(ws, 0, ((size_t)NA + NB) * sizeof(unsigned long long), st));
+    // precision 2: persistent correlation kernel; its split launch zeroes the keys, and the mutual test and the compaction
+    // are one kernel.  Empty inputs take the memset / flag / compact path below (count 0).
+    const bool pipe = precision == 2 && NA > 0 && NB > 0;
+    if (!pipe) RF_CUDA(cudaMemsetAsync(ws, 0, ((size_t)NA + NB) * sizeof(unsigned long long), st));
     if (NA > 0 && NB > 0) {
         RF_REQUIRE(precision >= 0 && precision <= 2, "rf_corr_mutual_nn: precision is 0 (fp32 SIMT), 1 (3xTF32) or 2 (fp16 split)");
         if (precision >= 1) {
-            int rc = rf_corr_argmax_tc(featA, NA, featB, NB, C, rowbest, colbest, static_cast<unsigned char*>(ws) + keys_bytes(NA, NB), st, precision, v2);
+            int rc = rf_corr_argmax_tc(featA, NA, featB, NB, C, rowbest, colbest, static_cast<unsigned char*>(ws) + keys_bytes(NA, NB), st, precision);
             if (rc) return rc;
         } else {
             dim3 grid((NB + 127) / 128, (NA + BM - 1) / BM);
@@ -560,7 +557,7 @@ extern "C" int rf_corr_mutual_nn(const float* featA, int NA, const float* featB,
             RF_LAUNCHED();
         }
     }
-    if (v2) return launch_mutual_compact(rowbest, colbest, NA, NB, (long long*)idx1_out, (long long*)idx2_out, count_out, st);
+    if (pipe) return launch_mutual_compact(rowbest, colbest, NA, NB, (long long*)idx1_out, (long long*)idx2_out, count_out, st);
     if (NA > 0) {
         mutual_flag_kernel<<<(NA + 255) / 256, 256, 0, st>>>(rowbest, colbest, NA);
         RF_LAUNCHED();
@@ -581,21 +578,13 @@ extern "C" int rf_corr_mutual_nn_presplit(const void* A_hi, const void* A_lo, in
     cudaStream_t st = as_stream(stream);
     unsigned long long* rowbest = reinterpret_cast<unsigned long long*>(ws);
     unsigned long long* colbest = rowbest + NA;
-    RF_CUDA(cudaMemsetAsync(ws, 0, ((size_t)NA + NB + 1) * sizeof(unsigned long long), st));       // keys + the tail's ticket counter
+    RF_CUDA(cudaMemsetAsync(ws, 0, ((size_t)NA + NB) * sizeof(unsigned long long), st));
     if (NA == 0 || NB == 0) {
         RF_CUDA(cudaMemsetAsync(count_out, 0, sizeof(int), st));
         return 0;
     }
     const void* planes[4] = {A_hi, A_lo, B_hi, B_lo};
-    // RF_CORR_TAIL=1: mutual test + compaction in the correlation kernel's last CTA (2 graph nodes instead of 3).  Measured
-    // SLOWER at config 2 (92.3 vs 86.5 us per call: 192 threads of one CTA do serially what the 1024-thread kernel does
-    // while nothing else is left to overlap with), so the separate column-driven kernel stays the default.
-    const char* e = getenv("RF_CORR_TAIL");
-    if ((e ? atoi(e) : 0) && NA <= 49152) {
-        void* tail[4] = {idx1_out, idx2_out, count_out, colbest + NB};
-        return rf_corr_argmax_tc(nullptr, NA, nullptr, NB, C, rowbest, colbest, nullptr, st, 2, true, planes, tail);
-    }
-    int rc = rf_corr_argmax_tc(nullptr, NA, nullptr, NB, C, rowbest, colbest, nullptr, st, 2, true, planes);
+    int rc = rf_corr_argmax_tc(nullptr, NA, nullptr, NB, C, rowbest, colbest, nullptr, st, 2, planes);
     if (rc) return rc;
     return launch_mutual_compact(rowbest, colbest, NA, NB, (long long*)idx1_out, (long long*)idx2_out, count_out, st);
 }

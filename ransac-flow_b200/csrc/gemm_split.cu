@@ -23,7 +23,6 @@
 //               (+ residual hi + lo * 2^-11, TMA-loaded into the group's staging buffer by its own leader) -> ReLU -> split ->
 //               swizzled staging [hi box | lo box] -> one TMA store.
 //               `out32`: fp32 rows straight to global memory instead (the 49- / 1-channel outputs of the heads).
-#include <cstdlib>
 
 #include "common.cuh"
 #include "tc_common.cuh"
@@ -31,7 +30,8 @@
 namespace rf {
 
 constexpr int SP_BN = 64;
-constexpr int sp_threads(int epw) { return 64 + 2 * 32 * epw; }          // producer warp + MMA warp + two epilogue groups of `epw` warps
+constexpr int SP_EPW = 8;                                                   // warps per epilogue group
+constexpr int SP_THREADS = 64 + 2 * 32 * SP_EPW;                            // producer warp + MMA warp + two epilogue groups
 constexpr int SP_HALO_TW = 8, SP_HALO_TH = 16, SP_HALO_LD = SP_HALO_TW + 2;
 constexpr int SP_HALO_PLANE = SP_HALO_LD * (SP_HALO_TH + 2) * 128;          // 23040 B: one plane of a halo block
 
@@ -52,7 +52,6 @@ struct alignas(64) SplitParams {
     int R, S, pad, stride, Cin, Cout, relu, has_res, out32;
     int tiles_m, tiles_n;
     int kc1, stride2;                     // dual-input 1x1: K blocks [0, kc1) come from mapA, the rest from mapR (second input, its own stride)
-    int dbg;                              // timing experiments only (RF_SPLIT_DBG): 1 no B loads, 2 no MMAs, 4 no A loads, 8 no epilogue math / store, 16 three MMAs per K step instead of two
     const float* bias;
     float* y32;                           // out32: fp32 [P][Cout]
 };
@@ -157,12 +156,11 @@ __device__ __forceinline__ void sp_split2(float a, float b, __half2& hi, __half2
     lo = sp_pack_sat((a - f.x) * 2048.f, (b - f.y) * 2048.f);
 }
 
-template <bool HALO, int BN_, bool RES2 = false, int EPW = 8>
-__global__ void __launch_bounds__(sp_threads(EPW), 1)
+template <bool HALO, int BN_, bool RES2 = false>
+__global__ void __launch_bounds__(SP_THREADS, 1)
 tc_split_kernel(const __grid_constant__ SplitParams p) {
     using Cfg = SplitCfg<HALO, BN_, RES2>;
-    static_assert(EPW == 4 || EPW == 8, "epilogue warps per group");
-    constexpr int GT = 32 * EPW;                // threads of one epilogue group
+    constexpr int GT = 32 * SP_EPW;             // threads of one epilogue group
     constexpr int NSB = Cfg::NSB;
     constexpr int BN = Cfg::BN, NA = Cfg::NA, NB = Cfg::NB, TB = Cfg::TB, BK = TC_BK_F16;
     constexpr bool WIDE = BN == 128;            // both epilogue groups work on every tile (one 64-channel half each)
@@ -209,10 +207,7 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
                     const int sa = ia_cnt % NA;
                     mbar_wait(&emptyA[sa], ((ia_cnt / NA) & 1) ^ 1);
                     int tap = 0, cc = ia;
-                    if (p.dbg & 4) {
-                        if (!HALO) { tap = ia / kc; cc = ia - tap * kc; }
-                        mbar_arrive(&fullA[sa]);
-                    } else if (HALO) {
+                    if (HALO) {
                         mbar_expect_tx(&fullA[sa], Cfg::A_TX);
                         tma_load_4d(sA + sa * Cfg::A_SLOT, &p.mapA[c.img], &fullA[sa], ia * BK, c.ox0 - 1, c.oy0 - 1, 0);
                     } else {
@@ -229,7 +224,6 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
                     for (int jb = 0; jb < TB; ++jb, ++ib_cnt) {
                         const int sb = ib_cnt % NB;
                         mbar_wait(&emptyB[sb], ((ib_cnt / NB) & 1) ^ 1);
-                        if (p.dbg & 1) { mbar_arrive(&fullB[sb]); continue; }
                         mbar_expect_tx(&fullB[sb], Cfg::B_TILE);
                         const int btap = HALO ? jb : tap;
                         tma_load_3d(sB + sb * Cfg::B_TILE, &p.mapB, &fullB[sb], btap * p.Cin + cc * BK, c.n0, 0);
@@ -245,7 +239,7 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
             const uint32_t buf = ti & 1;
             mbar_wait(&tmem_empty[buf], ((ti >> 1) & 1) ^ 1);               // the epilogue has drained this accumulator pair
             tc_fence_after();
-            const uint32_t td = tmem_base + buf * (2 * BN), tx = td + BN;
+            const uint32_t td = tmem_base + buf * (2 * BN);
             for (int ia = 0; ia < NAI; ++ia, ++ia_cnt) {
                 const int sa = ia_cnt % NA;
                 mbar_wait(&fullA[sa], (ia_cnt / NA) & 1);
@@ -260,12 +254,8 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
                     if (HALO) { const int r = jb / 3, sx = jb - r * 3; aaddr += (uint32_t)((r * SP_HALO_LD + sx) * 128); }
                     const uint64_t ahi = HALO ? sp_desc_halo(aaddr) : make_desc_sw128(aaddr);
                     const uint64_t alo = HALO ? sp_desc_halo(aaddr + Cfg::A_LO) : make_desc_sw128(aaddr + Cfg::A_LO);
-                    if (p.dbg & 2) {
-                    } else if (p.dbg & 16) {         // three N-wide MMAs per step (the first version; kept for A/B timing)
-                        umma_f16split_x4(td, tx, ahi, alo, make_desc_sw128(bb), make_desc_sw128(bb + Cfg::B_PLANE), idesc, (ia | jb) != 0 ? 1u : 0u);
-                    } else {                         // [B hi | B lo] as one 2N-wide instruction + A lo x B hi
-                        umma_f16split2_x4(td, BN, ahi, alo, make_desc_sw128(bb), make_idesc_f16(2 * BN), idesc, (ia | jb) != 0 ? 1u : 0u);
-                    }
+                    // [B hi | B lo] as one 2N-wide instruction + A lo x B hi
+                    umma_f16split2_x4(td, BN, ahi, alo, make_desc_sw128(bb), make_idesc_f16(2 * BN), idesc, (ia | jb) != 0 ? 1u : 0u);
                     umma_commit(&emptyB[sb]);
                 }
                 umma_commit(&emptyA[sa]);
@@ -274,17 +264,16 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
         }
     } else {
         // =============================== epilogue groups ===============================
-        // A group is EPW warps.  EPW = 4: one warp per TMEM lane quarter, 64 columns each; EPW = 8: two warps per quarter, 32
-        // columns each - the epilogue is ~11 fp32 instructions per output element (combine, bias, residual hi + lo, ReLU, split)
-        // in dependent chains, and with K <= 256 it, not the MMAs or HBM, sets the tile rate (ncu: 2.5 warps per scheduler,
-        // 6.2 cycles between issues); sixteen epilogue warps halve the drain time of an accumulator pair.
-        const uint32_t g = (uint32_t)(warp - 2) / EPW;                      // group 0 / 1
-        const int idx = (warp - 2) % EPW;
+        // A group is eight warps: two warps per TMEM lane quarter, 32 columns each - the epilogue is ~11 fp32 instructions per
+        // output element (combine, bias, residual hi + lo, ReLU, split) in dependent chains, and with K <= 256 it, not the MMAs
+        // or HBM, sets the tile rate (ncu: 2.5 warps per scheduler, 6.2 cycles between issues); sixteen epilogue warps halve the
+        // drain time of an accumulator pair against one warp per quarter.
+        const uint32_t g = (uint32_t)(warp - 2) / SP_EPW;                   // group 0 / 1
+        const int idx = (warp - 2) % SP_EPW;
         const int q = warp & 3;                                             // TMEM lane quarter this warp may access
         const int m = q * 32 + lane;
         const bool leader = idx == 0 && lane == 0;
-        constexpr int NCB = EPW == 8 ? 1 : 2;                               // 32-column blocks per thread
-        const int cb0 = EPW == 8 ? (idx >> 2) : 0;
+        const int cb = idx >> 2;                                            // this warp's 32-column block
         uint8_t* stg_base = sStg + g * NSB * Cfg::STG;
         uint32_t k = 0;                                                     // this group's tile counter
         const int t_first = blockIdx.x + (WIDE ? 0 : (int)g * (int)gridDim.x), t_step = (WIDE ? 1 : 2) * (int)gridDim.x;
@@ -331,9 +320,7 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
             }
             const uint32_t trow = tmem_base + buf * (2 * BN) + (WIDE ? 64 * g : 0) + ((uint32_t)(q * 32) << 16);
             float* yrow = p.out32 ? p.y32 + pix * p.Cout : nullptr;
-#pragma unroll 1
-            for (int cbi = 0; cbi < ((p.dbg & 8) ? 0 : NCB); ++cbi) {
-                const int cb = cb0 + cbi;
+            {
                 uint32_t v[32], x[32];
                 tmem_ld32x2(trow + cb * 32, v, trow + BN + cb * 32, x);
                 const int n = nbase + cb * 32;
@@ -393,7 +380,7 @@ tc_split_kernel(const __grid_constant__ SplitParams p) {
                 fence_proxy_async();
                 group_sync();
                 if (leader) {
-                    if (nbase < p.Cout && !(p.dbg & 8)) tma_store_4d(&p.mapY[c.img], stg, nbase, c.ox0, c.oy0, 0);
+                    if (nbase < p.Cout) tma_store_4d(&p.mapY[c.img], stg, nbase, c.ox0, c.oy0, 0);
                     if (RES2) {
                         asm volatile("cp.async.bulk.commit_group;" ::: "memory");   // read out while the group works on its next tile
                     } else {
@@ -753,27 +740,16 @@ static int rf_conv2d_split_impl(const ImgSet& set, const ConvParams& cp, const v
     }
     for (int i = set.n; i <= RF_MAX_IMGS; ++i) p.tile_start[i] = tiles;
     p.out_pix[set.n] = set.out_pix[set.n];
-    // 128-channel tiles for the tap-streaming layers that have them (RF_SPLIT_BN=64 forces the narrow tile everywhere)
-    static int bn_env = -1;
-    if (bn_env < 0) { const char* e = getenv("RF_SPLIT_BN"); bn_env = e ? atoi(e) : 128; }
     // measured per layer (profiles/r2_*): wide tiles pay for deep-K layers with >= 2 channel tiles and no residual (ResNet
     // down-sampling 1x1s, bottleneck c1 of layer 3, the stride-2 3x3s): -7 .. -15 %; the residual layers and 128-channel outputs
     // are faster with narrow tiles taken alternately by the two epilogue groups
-    static int shallow_env = -1;
-    if (shallow_env < 0) { const char* e = getenv("RF_SPLIT_SHALLOW"); shallow_env = e ? atoi(e) : 1; }
     // ONE K block per tile and no residual (two K blocks - the fused conv3 + down-sampling of layer1 - need both operand slots of
     // that variant for one tile, which serialises load latency and MMAs: 116 us against 85 us with the wide tile): the epilogue sets the tile rate, and the double-buffered-staging variant
     // (64-channel tiles, store read-out off the critical path) beats the wide tile (ResNet layer1 down-sampling 1x1: 79 -> 75 us)
-    const bool shallow = !halo && cp.R == 1 && cp.K <= 64 && shallow_env != 0;
-    static int halo_bn_env = -1;
-    if (halo_bn_env < 0) { const char* e = getenv("RF_SPLIT_HALO_BN"); halo_bn_env = e ? atoi(e) : 128; }
+    const bool shallow = !halo && cp.R == 1 && cp.K <= 64;
     // halo reuse with 128-channel tiles (N = 128 MMAs: less issue overhead per MAC, half the halo-block traffic; two-deep weight ring)
-    const bool halo_wide = halo && halo_bn_env == 128 && cp.Cout >= 128 && (cp.Cout % 128) == 0;
-    static int bn_min_env = -1, res_bn_env = -1;
-    if (bn_min_env < 0) { const char* e = getenv("RF_SPLIT_BN_MIN"); bn_min_env = e ? atoi(e) : 256; }
-    if (res_bn_env < 0) { const char* e = getenv("RF_SPLIT_RES_BN"); res_bn_env = e ? atoi(e) : 128; }
-    const bool tap_wide = !halo && !shallow && bn_env == 128 && (cp.Cout % 128) == 0 &&
-                          (cp.residual == nullptr ? cp.Cout >= bn_min_env : (res_bn_env == 128 && cp.K > 128));
+    const bool halo_wide = halo && cp.Cout >= 128 && (cp.Cout % 128) == 0;
+    const bool tap_wide = !halo && !shallow && (cp.Cout % 128) == 0 && (cp.residual == nullptr ? cp.Cout >= 256 : cp.K > 128);
     const int BN = (halo_wide || tap_wide) ? 128 : 64;
     int rc = get_map(&p.mapB, w_split, (unsigned long long)cp.K, (unsigned long long)cp.Cout, 2, TC_BK_F16, (unsigned)BN, 2, 1, 2);
     if (rc) return rc;
@@ -785,9 +761,6 @@ static int rf_conv2d_split_impl(const ImgSet& set, const ConvParams& cp, const v
     p.out32 = out32 ? 1 : 0;
     p.bias = cp.bias;
     p.y32 = out32 ? cp.y : nullptr;
-    static int dbg_env = -1;
-    if (dbg_env < 0) { const char* e = getenv("RF_SPLIT_DBG"); dbg_env = e ? atoi(e) : 0; }
-    p.dbg = dbg_env;
 
     p.tiles_m = tiles;
     p.tiles_n = (cp.Cout + BN - 1) / BN;
@@ -795,37 +768,26 @@ static int rf_conv2d_split_impl(const ImgSet& set, const ConvParams& cp, const v
     const long long total = (long long)p.tiles_m * p.tiles_n;
     RF_REQUIRE(total < (1ll << 24), "rf_conv2d_nhwc: too many tiles");          // sp_fast_div is exact below 2^24
     const int grid = total < num_sms() ? (int)total : num_sms();
-    static int res2_env = -1, epw_env = -1;
-    if (res2_env < 0) { const char* e = getenv("RF_SPLIT_RES2"); res2_env = e ? atoi(e) : 1; }
-    if (epw_env < 0) { const char* e = getenv("RF_SPLIT_EPW"); epw_env = (e && atoi(e) == 4) ? 4 : 8; }
     // double-buffered staging pays for the HBM-bound residual layers with one or two K blocks per tile (ResNet layer 1 / 2
     // c3 + residual: 147 -> 121 us, 81 -> 64 us); with four K blocks (layer 3) the 2-deep operand ring costs more than the
     // residual prefetch gains (45 -> 52 us): measured, profiles/README.md
-    const int which = halo ? (halo_wide ? 4 : 1) : (BN == 128 ? 2 : ((((cp.residual != nullptr && cp.K <= 128) || shallow) && res2_env) ? 3 : 0));
+    const int which = halo ? (halo_wide ? 4 : 1) : (BN == 128 ? 2 : (((cp.residual != nullptr && cp.K <= 128) || shallow) ? 3 : 0));
     const int dev = current_device();
-    static bool attr[64][10] = {{false}};
-    auto launch = [&](auto kernel, int smem, int threads, int slot) -> int {
+    static bool attr[64][5] = {{false}};
+    auto launch = [&](auto kernel, int smem, int slot) {
         if (!attr[dev][slot]) {
             RF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             attr[dev][slot] = true;
         }
-        kernel<<<grid, threads, smem, st>>>(p);
+        kernel<<<grid, SP_THREADS, smem, st>>>(p);
         return 0;
     };
     int lrc;
-    if (epw_env == 8) {
-        if (which == 4) lrc = launch(tc_split_kernel<true, 128, false, 8>, SplitCfg<true, 128>::SMEM_BYTES, sp_threads(8), 8);
-        else if (which == 1) lrc = launch(tc_split_kernel<true, 64, false, 8>, SplitCfg<true, 64>::SMEM_BYTES, sp_threads(8), 0);
-        else if (which == 2) lrc = launch(tc_split_kernel<false, 128, false, 8>, SplitCfg<false, 128>::SMEM_BYTES, sp_threads(8), 1);
-        else if (which == 3) lrc = launch(tc_split_kernel<false, 64, true, 8>, SplitCfg<false, 64, true>::SMEM_BYTES, sp_threads(8), 2);
-        else lrc = launch(tc_split_kernel<false, 64, false, 8>, SplitCfg<false, 64>::SMEM_BYTES, sp_threads(8), 3);
-    } else {
-        if (which == 4) lrc = launch(tc_split_kernel<true, 128, false, 4>, SplitCfg<true, 128>::SMEM_BYTES, sp_threads(4), 9);
-        else if (which == 1) lrc = launch(tc_split_kernel<true, 64, false, 4>, SplitCfg<true, 64>::SMEM_BYTES, sp_threads(4), 4);
-        else if (which == 2) lrc = launch(tc_split_kernel<false, 128, false, 4>, SplitCfg<false, 128>::SMEM_BYTES, sp_threads(4), 5);
-        else if (which == 3) lrc = launch(tc_split_kernel<false, 64, true, 4>, SplitCfg<false, 64, true>::SMEM_BYTES, sp_threads(4), 6);
-        else lrc = launch(tc_split_kernel<false, 64, false, 4>, SplitCfg<false, 64>::SMEM_BYTES, sp_threads(4), 7);
-    }
+    if (which == 4) lrc = launch(tc_split_kernel<true, 128>, SplitCfg<true, 128>::SMEM_BYTES, 4);
+    else if (which == 1) lrc = launch(tc_split_kernel<true, 64>, SplitCfg<true, 64>::SMEM_BYTES, 0);
+    else if (which == 2) lrc = launch(tc_split_kernel<false, 128>, SplitCfg<false, 128>::SMEM_BYTES, 1);
+    else if (which == 3) lrc = launch(tc_split_kernel<false, 64, true>, SplitCfg<false, 64, true>::SMEM_BYTES, 2);
+    else lrc = launch(tc_split_kernel<false, 64>, SplitCfg<false, 64>::SMEM_BYTES, 3);
     if (lrc) return lrc;
     RF_LAUNCHED();
     return 0;

@@ -49,11 +49,6 @@ struct alignas(64) TcParams {
     float* y;
     unsigned long long* rowbest;          // MODE_CORR
     unsigned long long* colbest;
-    // tc_corr_pipe_kernel, optional fused tail: the last CTA to finish runs the mutual test + order-preserving compaction
-    unsigned int* done_counter;           // zeroed by the caller with the keys
-    long long* tail_idx1;                 // nullptr: no tail
-    long long* tail_idx2;
-    int* tail_count;
     int NA, NB;
 };
 
@@ -237,9 +232,8 @@ tc_kernel(const __grid_constant__ TcParams p) {
     using Cfg = TcCfg<BN, MODE, DEEP>;
     constexpr int STAGES = Cfg::STAGES, NSPLIT = Cfg::NSPLIT;
     constexpr int BK = tc_bk<F16>();              // channels per 128-byte K block
-    constexpr bool CORR16 = F16 && MODE == MODE_CORR;                 // correlation with fp16-split operands: two accumulators
-    constexpr int TMEM_COLS = CORR16 ? 2 * Cfg::TMEM_COLS : Cfg::TMEM_COLS;
-    static_assert(TMEM_COLS <= 512, "TMEM");
+    constexpr int TMEM_COLS = Cfg::TMEM_COLS;
+    static_assert(!(F16 && MODE == MODE_CORR), "the fp16-split correlation is tc_corr_pipe_kernel");
     // fp16 convolutions: ring depth per layer (<= STAGES) and, for layers with a residual, a dedicated staging area
     // behind the ring that the producer fills at CTA start (more bytes in flight per SM, one DRAM latency less per CTA)
     const int NST = (F16 && MODE == MODE_CONV) ? p.stages : STAGES;
@@ -326,9 +320,7 @@ tc_kernel(const __grid_constant__ TcParams p) {
                 const uint32_t sa = smem_u32(smem + st * Cfg::STAGE_BYTES);
                 const uint32_t sb = sa + NSPLIT * TC_A_BYTES;
                 const uint64_t da = make_desc_sw128(sa), db = make_desc_sw128(sb);
-                if (CORR16) {
-                    umma_f16split_x4(tmem_base, tmem_base + BN, da, make_desc_sw128(sa + TC_A_BYTES), db, make_desc_sw128(sb + Cfg::B_BYTES), idesc, it != 0 ? 1u : 0u);
-                } else if (NSPLIT == 2) {
+                if (NSPLIT == 2) {
                     umma_3xtf32_x4(tmem_base, da, make_desc_sw128(sa + TC_A_BYTES), db, make_desc_sw128(sb + Cfg::B_BYTES), idesc, it != 0 ? 1u : 0u);
                 } else {
                     umma_x4<F16>(tmem_base, da, db, idesc, it != 0 ? 1u : 0u);      // 4 x (UMMA_K = 8 tf32 / 16 fp16 = 32 bytes)
@@ -358,12 +350,6 @@ tc_kernel(const __grid_constant__ TcParams p) {
             for (int c = 0; c < BN / 32; ++c) {
                 uint32_t v[32];
                 tmem_ld32(trow + c * 32, v);
-                if (CORR16) {                       // + the cross terms, accumulated at 2^11 scale in the second accumulator
-                    uint32_t x[32];
-                    tmem_ld32(trow + BN + c * 32, x);
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) v[j] = __float_as_uint(fmaf(__uint_as_float(x[j]), 0.00048828125f, __uint_as_float(v[j])));
-                }
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     const int col = n0 + c * 32 + j;
@@ -422,7 +408,7 @@ struct HaloCfg {
     static constexpr int TMEM_COLS = BN <= 64 ? 64 : 128;
 };
 
-__device__ __forceinline__ uint64_t make_desc_halo(uint32_t saddr, int mode) {
+__device__ __forceinline__ uint64_t make_desc_halo(uint32_t saddr) {
     uint64_t d = 0;
     d |= (uint64_t)(saddr >> 4);
     d |= (uint64_t)1 << 16;
@@ -432,7 +418,6 @@ __device__ __forceinline__ uint64_t make_desc_halo(uint32_t saddr, int mode) {
     // 128-byte swizzle of tcgen05.mma is a pure function of the shared-memory address bits (it matches what the TMA
     // wrote for any row phase) and the descriptor's base-offset field must stay 0; setting it to (addr >> 7) & 7, as the
     // PTX text suggests for unaligned starts, double-applies the phase and gives wrong results.
-    (void)mode;
     d |= (uint64_t)2 << 61;
     return d;
 }
@@ -440,7 +425,7 @@ __device__ __forceinline__ uint64_t make_desc_halo(uint32_t saddr, int mode) {
 // OUT32 (with F16): fp16 operands, fp32 output through the fp32 epilogue (the layer feeding a TF32 / fp32 consumer)
 template <int BN, bool F16 = false, bool OUT32 = false>
 __global__ void __launch_bounds__(TC_THREADS, 2)
-tc_halo_kernel(const __grid_constant__ TcParams p, int desc_mode) {
+tc_halo_kernel(const __grid_constant__ TcParams p) {
     using Cfg = HaloCfg<BN>;
     constexpr int NA = Cfg::NA, NB = Cfg::NB;
     constexpr int BK = tc_bk<F16>();
@@ -512,7 +497,7 @@ tc_halo_kernel(const __grid_constant__ TcParams p, int desc_mode) {
                     const int r = tap / 3, sx = tap - r * 3;
                     const uint32_t aaddr = abase + (uint32_t)((r * HALO_LD + sx) * 128);
                     const uint64_t db = make_desc_sw128(smem_u32(sB + sb * Cfg::B_BYTES));
-                    umma_x4<F16>(tmem_base, make_desc_halo(aaddr, desc_mode), db, idesc, (cc | tap) != 0 ? 1u : 0u);
+                    umma_x4<F16>(tmem_base, make_desc_halo(aaddr), db, idesc, (cc | tap) != 0 ? 1u : 0u);
                     umma_commit(&emptyB[sb]);
                 }
                 umma_commit(&emptyA[sa]);
@@ -532,33 +517,8 @@ tc_halo_kernel(const __grid_constant__ TcParams p, int desc_mode) {
 }
 
 
-// ------------------------------------------------------------------------------------------------------------
-// PERSISTENT convolution kernel: one CTA per SM walks a static list of tiles.  Most layers of this workload have a
-// short K loop (1x1 convs: 2-32 steps; 3x3 on 64 channels: 2 halo chunks), so a one-tile-per-CTA kernel spends its
-// life in prologue / TMA round-trip / epilogue latency.  Here the three roles run decoupled across tiles:
-//   warp 0   : TMA producer - keeps the A ring (tap tiles, or halo chunks when HALO) and the B ring (weight tiles)
-//              full, running ahead into the next tile while the current one is multiplied;
-//   warp 1   : MMA issuer - two TMEM accumulators (2 x BN columns): tile i+1 accumulates while tile i drains;
-//   warps 2-5: epilogue - TMEM -> (+bias, +residual, ReLU, TF32 round) -> swizzled smem staging -> TMA store, two
-//              staging buffers so the residual tile of tile i+1 is prefetched while tile i is being stored.
-// ------------------------------------------------------------------------------------------------------------
-template <int BN, bool HALO>
-struct PCfg {
-    static constexpr int A_SLOT = HALO ? HALO_A_SLOT : TC_A_BYTES;
-    static constexpr int A_TX = HALO ? HALO_A_BYTES : TC_A_BYTES;
-    static constexpr int B_BYTES = BN * 128;
-    static constexpr int NA = HALO ? 2 : (BN == 128 ? 3 : 4);
-    static constexpr int NB = HALO ? (BN == 128 ? 3 : 6) : NA;
-    static constexpr int STG = BN * 512;
-    static constexpr int OFF_B = NA * A_SLOT;
-    static constexpr int OFF_STG = OFF_B + NB * B_BYTES;
-    static constexpr int DATA_BYTES = OFF_STG + 2 * STG;
-    static constexpr int SMEM_BYTES = DATA_BYTES + 1024 + 512;
-    static constexpr int TMEM_COLS = 2 * BN;
-    static constexpr int TB = HALO ? 9 : 1;                 // B tiles consumed per A slot
-};
-
-
+// Tile decode of the persistent convolution kernels (tc_resb_kernel, tc_pipe_kernel): tile t of tiles_m pixel tiles x
+// (Cout / BN) channel tiles.
 struct TileCoord { int img, ox0, oy0, tw, n0; };
 
 template <bool HALO>
@@ -583,169 +543,6 @@ __device__ __forceinline__ TileCoord decode_tile(const TcParams& p, int t, int t
     c.n0 = nt * BN;
     return c;
 }
-
-template <int BN, bool HALO>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-tc_persist_kernel(const __grid_constant__ TcParams p, int tiles_m, int tiles_n) {
-    using Cfg = PCfg<BN, HALO>;
-    constexpr int NA = Cfg::NA, NB = Cfg::NB, TB = Cfg::TB;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);      // pointer arithmetic keeps the shared address space (LDS / STS, not generic LD / ST)
-    uint8_t* sA = smem;
-    uint8_t* sB = smem + Cfg::OFF_B;
-    uint8_t* sStg = smem + Cfg::OFF_STG;
-    uint64_t* fullA = reinterpret_cast<uint64_t*>(smem + Cfg::DATA_BYTES);
-    uint64_t* emptyA = fullA + NA;
-    uint64_t* fullB = emptyA + NA;
-    uint64_t* emptyB = fullB + NB;
-    uint64_t* tmem_full = emptyB + NB;          // [2]
-    uint64_t* tmem_empty = tmem_full + 2;       // [2]
-    uint64_t* res_full = tmem_empty + 2;        // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_full + 2);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int total = tiles_m * tiles_n;
-    const int kc = p.Cin / TC_BK;
-    const int NAI = HALO ? kc : p.R * p.S * kc;             // A slots per tile
-
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < NA; ++i) { mbar_init(&fullA[i], 1); mbar_init(&emptyA[i], 1); }
-        for (int i = 0; i < NB; ++i) { mbar_init(&fullB[i], 1); mbar_init(&emptyB[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 128); mbar_init(&res_full[i], 1); }
-        fence_barrier_init();
-    }
-    if (warp == 0 && lane == 0) { tma_prefetch_desc(&p.mapA[0]); tma_prefetch_desc(&p.mapB); tma_prefetch_desc(&p.mapY[0]); }
-    if (warp == 1) tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        // =============================== TMA producer ===============================
-        if (lane == 0) {
-            uint32_t ia_cnt = 0, ib_cnt = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                const TileCoord c = decode_tile<HALO>(p, t, tiles_m, BN);
-                for (int ia = 0; ia < NAI; ++ia, ++ia_cnt) {
-                    const int sa = ia_cnt % NA;
-                    mbar_wait(&emptyA[sa], ((ia_cnt / NA) & 1) ^ 1);
-                    mbar_expect_tx(&fullA[sa], Cfg::A_TX);
-                    int tap = 0, cc = ia;
-                    if (HALO) {
-                        tma_load_3d(sA + sa * Cfg::A_SLOT, &p.mapA[c.img], &fullA[sa], ia * TC_BK, c.ox0 - 1, c.oy0 - 1);
-                    } else {
-                        tap = ia / kc;
-                        cc = ia - tap * kc;
-                        const int r = tap / p.S, sx = tap - r * p.S;
-                        tma_load_3d(sA + sa * Cfg::A_SLOT, &p.mapA[c.img], &fullA[sa], cc * TC_BK, c.ox0 * p.stride + sx - p.pad,
-                                    c.oy0 * p.stride + r - p.pad);
-                    }
-                    for (int jb = 0; jb < TB; ++jb, ++ib_cnt) {
-                        const int sb = ib_cnt % NB;
-                        mbar_wait(&emptyB[sb], ((ib_cnt / NB) & 1) ^ 1);
-                        mbar_expect_tx(&fullB[sb], Cfg::B_BYTES);
-                        const int btap = HALO ? jb : tap;
-                        tma_load_2d(sB + sb * Cfg::B_BYTES, &p.mapB, &fullB[sb], btap * p.Cin + cc * TC_BK, c.n0);
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // =============================== MMA issuer ===============================
-        {   // whole warp, warp-uniform control flow; umma_* elect the issuing lane
-            constexpr uint32_t idesc = make_idesc_tf32(BN);
-            uint32_t ia_cnt = 0, ib_cnt = 0, ti = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x, ++ti) {
-                const uint32_t buf = ti & 1;
-                mbar_wait(&tmem_empty[buf], ((ti >> 1) & 1) ^ 1);       // the epilogue has drained this accumulator
-                tc_fence_after();
-                const uint32_t tacc = tmem_base + buf * BN;
-                for (int ia = 0; ia < NAI; ++ia, ++ia_cnt) {
-                    const int sa = ia_cnt % NA;
-                    mbar_wait(&fullA[sa], (ia_cnt / NA) & 1);
-                    tc_fence_after();
-                    const uint32_t abase = smem_u32(sA + sa * Cfg::A_SLOT);
-                    for (int jb = 0; jb < TB; ++jb, ++ib_cnt) {
-                        const int sb = ib_cnt % NB;
-                        mbar_wait(&fullB[sb], (ib_cnt / NB) & 1);
-                        tc_fence_after();
-                        const uint64_t db = make_desc_sw128(smem_u32(sB + sb * Cfg::B_BYTES));
-                        uint32_t aaddr = abase;
-                        if (HALO) { const int r = jb / 3, sx = jb - r * 3; aaddr += (uint32_t)((r * HALO_LD + sx) * 128); }
-                        umma_tf32_x4(tacc, HALO ? make_desc_halo(aaddr, 2) : make_desc_sw128(aaddr), db, idesc, (ia | jb) != 0 ? 1u : 0u);
-                        umma_commit(&emptyB[sb]);
-                    }
-                    umma_commit(&emptyA[sa]);
-                }
-                umma_commit(&tmem_full[buf]);
-            }
-        }
-    } else {
-        // =============================== epilogue (warps 2..5) ===============================
-        const int q = warp & 3;
-        const int m = q * 32 + lane;
-        const bool leader = (warp == 2 && lane == 0);
-        const bool has_res = p.residual != nullptr;
-        if (leader && has_res && (int)blockIdx.x < total) {
-            const TileCoord c = decode_tile<HALO>(p, blockIdx.x, tiles_m, BN);
-            mbar_expect_tx(&res_full[0], (BN / 32) * TC_A_BYTES);
-#pragma unroll
-            for (int cb = 0; cb < BN / 32; ++cb) tma_load_3d(sStg + cb * TC_A_BYTES, &p.mapR[c.img], &res_full[0], c.n0 + cb * 32, c.ox0, c.oy0);
-        }
-        uint32_t ti = 0;
-        for (int t = blockIdx.x; t < total; t += gridDim.x, ++ti) {
-            const uint32_t buf = ti & 1;
-            const TileCoord c = decode_tile<HALO>(p, t, tiles_m, BN);
-            uint8_t* stg = sStg + buf * Cfg::STG;
-            asm volatile("bar.sync 1, 128;" ::: "memory");           // the leader's bookkeeping of the previous tile is done
-            mbar_wait(&tmem_full[buf], (ti >> 1) & 1);
-            tc_fence_after();
-            if (has_res) mbar_wait(&res_full[buf], (ti >> 1) & 1);
-            const uint32_t trow = tmem_base + buf * BN + ((uint32_t)(q * 32) << 16);
-#pragma unroll 1
-            for (int cb = 0; cb < BN / 32; ++cb) {
-                uint32_t v[32];
-                tmem_ld32(trow + cb * 32, v);
-                const int n = c.n0 + cb * 32;
-                uint8_t* rowp = stg + cb * TC_A_BYTES + m * 128;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    float4* sp = reinterpret_cast<float4*>(rowp + ((j ^ (m & 7)) << 4));
-                    float4 o = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                    if (p.bias && n + 4 * j < p.Cout) { float4 b = __ldg(reinterpret_cast<const float4*>(p.bias + n + 4 * j)); o.x += b.x; o.y += b.y; o.z += b.z; o.w += b.w; }
-                    if (has_res) { float4 rr = *sp; o.x += rr.x; o.y += rr.y; o.z += rr.z; o.w += rr.w; }
-                    if (p.relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
-                    if (p.round_out) { o.x = round_tf32(o.x); o.y = round_tf32(o.y); o.z = round_tf32(o.z); o.w = round_tf32(o.w); }
-                    *sp = o;
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(&tmem_empty[buf]);                            // accumulator drained (128 arrivals)
-            fence_proxy_async();
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-            if (leader) {
-#pragma unroll
-                for (int cb = 0; cb < BN / 32; ++cb)
-                    if (c.n0 + cb * 32 < p.Cout) tma_store_3d(&p.mapY[c.img], stg + cb * TC_A_BYTES, c.n0 + cb * 32, c.ox0, c.oy0);
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");      // the other staging buffer has been read out
-                const int tn = t + gridDim.x;
-                if (has_res && tn < total) {
-                    const TileCoord cn = decode_tile<HALO>(p, tn, tiles_m, BN);
-                    uint8_t* stn = sStg + (buf ^ 1) * Cfg::STG;
-                    mbar_expect_tx(&res_full[buf ^ 1], (BN / 32) * TC_A_BYTES);
-#pragma unroll
-                    for (int cb = 0; cb < BN / 32; ++cb) tma_load_3d(stn + cb * TC_A_BYTES, &p.mapR[cn.img], &res_full[buf ^ 1], cn.n0 + cb * 32, cn.ox0, cn.oy0);
-                }
-            }
-        }
-        if (leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
-}
-
 
 // ------------------------------------------------------------------------------------------------------------
 // 3x3 / stride-1 / 64 -> 64 channel convolutions (ResNet-50 layer1 conv2, FeatureExtractor layer1): K is only two
@@ -842,7 +639,7 @@ tc_resb_kernel(const __grid_constant__ TcParams p, int tiles_m) {
                         const int r = tap / 3, sx = tap - r * 3;
                         const uint32_t aaddr = abase + (uint32_t)((r * HALO_LD + sx) * 128);
                         const uint64_t db = make_desc_sw128(smem_u32(sB + (cc * Cfg::NTAP + tap) * Cfg::B_TILE));
-                        umma_x4<F16>(tacc, make_desc_halo(aaddr, 2), db, idesc, (cc | tap) != 0 ? 1u : 0u);
+                        umma_x4<F16>(tacc, make_desc_halo(aaddr), db, idesc, (cc | tap) != 0 ? 1u : 0u);
                     }
                     umma_commit(&emptyA[sa]);
                 }
@@ -1045,7 +842,7 @@ tc_pipe_kernel(const __grid_constant__ TcParams p, int tiles_m, int tiles_n) {
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// PERSISTENT correlation + mutual-NN kernel (utils/outil.py:34-37, precision 2 = fp16 split).  ncu on the
+// PERSISTENT correlation + mutual-NN kernel (utils/outil.py:34-37, precision 2 = fp16 split).  ncu on the former
 // one-tile-per-CTA kernel (profiles/r1_corr_f16_ncu.json): 17.8 us per 128 x 128 score tile for 6.3 us of MMAs - one
 // CTA per SM (192 KB of stages), so TMEM allocation, the first TMA round trip and the whole arg-max epilogue are
 // serial with the K loop.  Here one CTA per SM walks its tiles (N-tiles fastest: the CTAs sharing a featA slab run
@@ -1056,8 +853,8 @@ tc_pipe_kernel(const __grid_constant__ TcParams p, int tiles_m, int tiles_n) {
 //   warps 2-5 : epilogue.  Row arg-max thread-local straight from TMEM; column arg-max 32 columns at a time through
 //               a 128 x 33 float transposition buffer of its own (the stages are busy), four row quarters combined
 //               through 1 KB of keys, one atomicMax per column and per row of the tile as before.
-// Same arithmetic per score as tc_kernel<128, MODE_CORR, false, true> (same MMAs in the same order, same fma of the
-// cross-term accumulator), same (score, smallest index) ordering => identical match lists.
+// Per score: hi*hi into the main accumulator, lo*hi + hi*lo (at 2^11 scale) into the cross one, combined with one fma;
+// ties go to the smallest index.
 // ------------------------------------------------------------------------------------------------------------
 struct CorrPipeCfg {
     static constexpr int BN = 128;
@@ -1140,19 +937,16 @@ tc_corr_pipe_kernel(const __grid_constant__ TcParams p, int tiles_m, int tiles_n
             const uint32_t buf = ti & 1;
             mbar_wait(&tmem_empty[buf], ((ti >> 1) & 1) ^ 1);               // the epilogue has drained this accumulator pair
             tc_fence_after();
-            const uint32_t td = tmem_base + buf * (2 * BN), tx = td + BN;
+            const uint32_t td = tmem_base + buf * (2 * BN);
             for (int it = 0; it < KI; ++it, ++cnt) {
                 const int st = cnt % NS;
                 mbar_wait(&full[st], (cnt / NS) & 1);
                 tc_fence_after();
                 const uint32_t sa = smem_u32(smem + st * Cfg::STAGE_BYTES);
                 const uint32_t sb = sa + 2 * TC_A_BYTES;
-                if (p.stages == 3)      // RF_CORR_MMA3=1: three N = 128 instructions per K step (the first version; A/B timing)
-                    umma_f16split_x4(td, tx, make_desc_sw128(sa), make_desc_sw128(sa + TC_A_BYTES), make_desc_sw128(sb),
-                                     make_desc_sw128(sb + Cfg::B_BYTES), idesc, it != 0 ? 1u : 0u);
-                else                    // [B hi | B lo] are adjacent in the stage, [main | cross] in TMEM: one N = 256 instruction + A lo x B hi
-                    umma_f16split2_x4(td, BN, make_desc_sw128(sa), make_desc_sw128(sa + TC_A_BYTES), make_desc_sw128(sb),
-                                      make_idesc_f16(2 * BN), idesc, it != 0 ? 1u : 0u);
+                // [B hi | B lo] are adjacent in the stage, [main | cross] in TMEM: one N = 256 instruction + A lo x B hi
+                umma_f16split2_x4(td, BN, make_desc_sw128(sa), make_desc_sw128(sa + TC_A_BYTES), make_desc_sw128(sb),
+                                  make_idesc_f16(2 * BN), idesc, it != 0 ? 1u : 0u);
                 umma_commit(&empty[st]);
             }
             umma_commit(&tmem_full[buf]);
@@ -1212,56 +1006,8 @@ tc_corr_pipe_kernel(const __grid_constant__ TcParams p, int tiles_m, int tiles_n
         }
     }
     tc_fence_before();
-    if (p.tail_idx1 != nullptr) __threadfence();                // this thread's arg-max atomics are performed before the ticket below
     __syncthreads();
     if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
-    if (p.tail_idx1 == nullptr) return;
-    // ---- fused tail: utils/outil.py:38-43 (mutual test, S*S > 0, nonzero() order) by the LAST CTA to finish, on the idle ring.
-    // Same algorithm as mutual_cols_compact_kernel (gemm_simt.cu), six warps instead of 32: identical index lists.
-    __shared__ unsigned int s_last;
-    __shared__ int s_cnt[TC_THREADS / 32];
-    if (threadIdx.x == 0) s_last = (atomicAdd(p.done_counter, 1u) == gridDim.x - 1) ? 1u : 0u;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    int* sRow = reinterpret_cast<int*>(smem);                   // 0 = unmatched row, j + 1 = matched with column j
-    const int tid = threadIdx.x, NA = p.NA, NB = p.NB;
-    constexpr int NW = TC_THREADS / 32;
-    for (int i = tid; i < NA; i += TC_THREADS) sRow[i] = 0;
-    __syncthreads();
-    for (int j = tid; j < NB; j += TC_THREADS) {
-        const unsigned long long ck = __ldcg(p.colbest + j);
-        if (ck == 0ull) continue;
-        const uint32_t i = key_index(ck);
-        if (i >= (uint32_t)NA) continue;
-        const unsigned long long rk = __ldcg(p.rowbest + i);
-        const float v = key_value(rk);
-        if (rk != 0ull && key_index(rk) == (uint32_t)j && (__fmul_rn(v, v) > 0.f)) sRow[i] = j + 1;
-    }
-    __syncthreads();
-    const int chunk = (((NA + 31) / 32) + NW - 1) / NW * 32;    // rows per warp, a multiple of 32
-    const int begin = warp * chunk;
-    int cnt = 0;
-    for (int b = 0; b < chunk; b += 32) {
-        const int i = begin + b + lane;
-        cnt += __popc(__ballot_sync(0xffffffffu, i < NA && sRow[i] != 0));
-    }
-    if (lane == 0) s_cnt[warp] = cnt;
-    __syncthreads();
-    int off = 0, total_m = 0;
-    for (int w = 0; w < NW; ++w) { const int v = s_cnt[w]; off += (w < warp) ? v : 0; total_m += v; }
-    for (int b = 0; b < chunk; b += 32) {
-        const int i = begin + b + lane;
-        const int f = (i < NA) ? sRow[i] : 0;
-        const uint32_t bal = __ballot_sync(0xffffffffu, f != 0);
-        if (f) {
-            const int o = off + __popc(bal & ((1u << lane) - 1u));
-            p.tail_idx1[o] = i;
-            p.tail_idx2[o] = (long long)(f - 1);
-        }
-        off += __popc(bal);
-    }
-    if (tid == 0) *p.tail_count = total_m;
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1420,25 +1166,8 @@ __global__ void split_tf32_kernel(const float4* __restrict__ x, float4* __restri
     lo[i] = l;
 }
 
-// fp16 split for the correlation (precision 2): hi = fp16(x), lo = fp16((x - hi) * 2^11)
-__global__ void split_f16_kernel(const float4* __restrict__ x, uint2* __restrict__ hi, uint2* __restrict__ lo, long long n4) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n4) return;
-    const float4 v = __ldg(x + i);
-    const __half2 h0 = __floats2half2_rn(v.x, v.y), h1 = __floats2half2_rn(v.z, v.w);
-    const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
-    const __half2 l0 = __floats2half2_rn((v.x - f0.x) * 2048.f, (v.y - f0.y) * 2048.f);
-    const __half2 l1 = __floats2half2_rn((v.z - f1.x) * 2048.f, (v.w - f1.y) * 2048.f);
-    uint2 ho, lo2;
-    ho.x = *reinterpret_cast<const uint32_t*>(&h0); ho.y = *reinterpret_cast<const uint32_t*>(&h1);
-    lo2.x = *reinterpret_cast<const uint32_t*>(&l0); lo2.y = *reinterpret_cast<const uint32_t*>(&l1);
-    hi[i] = ho;
-    lo[i] = lo2;
-}
-
-// Both feature matrices in ONE launch (fp16 split as above; hi/lo of A then hi/lo of B are consecutive in the workspace),
-// and the arg-max keys zeroed by the first threads: replaces a memset node and two split launches in front of the
-// persistent correlation kernel.
+// fp16 split for the correlation (precision 2) of both feature matrices in ONE launch: hi = fp16(x), lo = fp16((x - hi) * 2^11);
+// hi/lo of A then hi/lo of B are consecutive in the workspace, and the arg-max keys are zeroed by the first threads.
 __global__ void split_f16_all_kernel(const float4* __restrict__ A, const float4* __restrict__ B, uint2* __restrict__ Ahi, uint2* __restrict__ Alo,
                                      uint2* __restrict__ Bhi, uint2* __restrict__ Blo, long long na4, long long nb4,
                                      unsigned long long* __restrict__ keys, long long nkeys) {
@@ -1541,45 +1270,12 @@ int pick_tw(int Ho, int Wo) {
     return best;
 }
 
-static int halo_mode() {
-    static int m = -1;
-    if (m < 0) {
-        const char* e = getenv("RF_TC_HALO");     // 0 = tap-streaming kernel, anything else = halo reuse (default)
-        m = (e && atoi(e) == 0) ? 0 : 2;
-    }
-    return m;
-}
-
-static int corr_tile_n() {
-    static int m = -1;
-    if (m < 0) {
-        const char* e = getenv("RF_CORR_BN");     // 128 (default) or 256; measured equal within 3 % (191 vs 185 us): the
-        m = e ? atoi(e) : 128;                    // kernel is shared-memory-bandwidth bound (A+B 8 KB per 64-cycle MMA), not L2 bound
-    }
-    return m;
-}
-
-static int persist_mode() {
-    static int m = -1;
-    if (m < 0) {
-        const char* e = getenv("RF_TC_PERSIST");
-        m = e ? atoi(e) : 0;
-    }
-    return m;
-}
-
+// Off by default: measured -2 % end to end (profiles/README.md), the extra staging costs a resident CTA.  Kept because
+// the kernel without this path compiles worse: ptxas moves the one-tile fp16 kernel's prologue off the uniform datapath
+// (80 -> 84 registers) and those kernels run 12 % slower.
 static int respf_mode() {
-    const char* e = getenv("RF_TC_RESPF");    // fp16 1x1 convs with a residual: prefetch the residual tile at CTA start.
-    return e ? atoi(e) : 0;                     // Measured (profiles/README.md): -2 % end to end - the extra staging costs a resident CTA
-}
-
-static int resb_mode() {
-    static int m = -1;
-    if (m < 0) {
-        const char* e = getenv("RF_TC_RESB");     // weights-resident persistent kernel for 64 -> 64 3x3 convs (default on);
-        m = e ? atoi(e) : 1;                      // a 3-slot / direct-store variant measured no faster (332 vs 320 us per pair)
-    }
-    return m;
+    const char* e = getenv("RF_TC_RESPF");    // fp16 1x1 convs with a residual: prefetch the residual tile at CTA start
+    return e ? atoi(e) : 0;
 }
 
 template <bool F16>
@@ -1594,16 +1290,6 @@ static int launch_resb(const TcParams& p, int tiles_m, cudaStream_t st) {
     tc_resb_kernel<F16><<<grid, TC_THREADS, ResBCfg<F16>::SMEM_BYTES, st>>>(p, tiles_m);
     RF_LAUNCHED();
     return 0;
-}
-
-static int raster_mode() {
-    const char* e = getenv("RF_TC_RASTER");    // 1 (default): channel tiles fastest for the tap-streaming conv kernels - the CTAs
-    return e ? atoi(e) : 1;                     // of one pixel tile run together (A once from HBM, whole output rows); +2 % per pair
-}
-
-static int pipe_mode() {
-    const char* e = getenv("RF_TC_PIPE");    // pipelined persistent kernel for the fp16 tap-streaming convs: 0 never, 1 always,
-    return e ? atoi(e) : 2;                     // 2 (default) where it measured faster: >= 4 K blocks and >= 2 tiles per SM
 }
 
 template <int BN>
@@ -1622,24 +1308,8 @@ static int launch_pipe(const TcParams& p, int tiles_m, int tiles_n, cudaStream_t
     return 0;
 }
 
-template <int BN, bool HALO>
-static int launch_persist(const TcParams& p, int tiles_m, int tiles_n, cudaStream_t st) {
-    using Cfg = PCfg<BN, HALO>;
-    static bool attr[64] = {false};
-    const int dev = current_device();
-    if (!attr[dev]) {
-        RF_CUDA(cudaFuncSetAttribute(tc_persist_kernel<BN, HALO>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        attr[dev] = true;
-    }
-    const int total = tiles_m * tiles_n;
-    const int grid = total < num_sms() ? total : num_sms();
-    tc_persist_kernel<BN, HALO><<<grid, TC_THREADS, Cfg::SMEM_BYTES, st>>>(p, tiles_m, tiles_n);
-    RF_LAUNCHED();
-    return 0;
-}
-
 template <int BN, bool F16 = false, bool OUT32 = false>
-static int launch_halo(const TcParams& p, int tiles, int ntiles_n, int mode, cudaStream_t st) {
+static int launch_halo(const TcParams& p, int tiles, int ntiles_n, cudaStream_t st) {
     using Cfg = HaloCfg<BN>;
     static bool attr[64] = {false};
     const int dev = current_device();
@@ -1647,7 +1317,7 @@ static int launch_halo(const TcParams& p, int tiles, int ntiles_n, int mode, cud
         RF_CUDA(cudaFuncSetAttribute(tc_halo_kernel<BN, F16, OUT32>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
         attr[dev] = true;
     }
-    tc_halo_kernel<BN, F16, OUT32><<<dim3(tiles, ntiles_n), TC_THREADS, Cfg::SMEM_BYTES, st>>>(p, mode);
+    tc_halo_kernel<BN, F16, OUT32><<<dim3(tiles, ntiles_n), TC_THREADS, Cfg::SMEM_BYTES, st>>>(p);
     RF_LAUNCHED();
     return 0;
 }
@@ -1707,16 +1377,16 @@ int rf_conv2d_tc(const ImgSet& set, const ConvParams& cp, const void* w_tc, cuda
     const unsigned bk = f16 ? TC_BK_F16 : TC_BK;
     const unsigned esz_y = (f16 && !out32) ? 2u : 4u;                // output (and residual) element size
     const unsigned bk_y = (f16 && !out32) ? TC_BK_F16 : TC_BK;
-    RF_REQUIRE(!out32 || (f16 && cp.R == 3 && cp.stride == 1 && cp.pad == 1 && cp.residual == nullptr && halo_mode() != 0),
+    RF_REQUIRE(!out32 || (f16 && cp.R == 3 && cp.stride == 1 && cp.pad == 1 && cp.residual == nullptr),
                "rf_conv2d_nhwc: engine 3 (fp16 operands, fp32 output) covers 3x3 / stride 1 / pad 1 layers without residual");
     const char* xb = reinterpret_cast<const char*>(cp.x);
     const char* rb = reinterpret_cast<const char*>(cp.residual);
     char* yb = reinterpret_cast<char*>(cp.y);
     p.nimg = set.n;
-    const int hmode = (cp.R == 3 && cp.stride == 1 && cp.pad == 1) ? halo_mode() : 0;
+    const bool halo = cp.R == 3 && cp.stride == 1 && cp.pad == 1;      // halo reuse (tc_halo_kernel, tc_resb_kernel)
     int tiles = 0;
     for (int i = 0; i < set.n; ++i) {
-        int tw = hmode ? HALO_TW : pick_tw(set.Ho[i], set.Wo[i]), th = 128 / tw;
+        int tw = halo ? HALO_TW : pick_tw(set.Ho[i], set.Wo[i]), th = 128 / tw;
         p.tw[i] = tw;
         p.tiles_x[i] = (set.Wo[i] + tw - 1) / tw;
         p.tile_start[i] = tiles;
@@ -1724,7 +1394,7 @@ int rf_conv2d_tc(const ImgSet& set, const ConvParams& cp, const void* w_tc, cuda
         p.Ho[i] = set.Ho[i]; p.Wo[i] = set.Wo[i];
         p.out_pix[i] = set.out_pix[i];
         int rc = get_map(&p.mapA[i], xb + set.in_pix[i] * cp.Cin * esz, (unsigned long long)cp.Cin, (unsigned long long)set.W[i],
-                         (unsigned long long)set.H[i], bk, (unsigned)(hmode ? tw + 2 : tw), (unsigned)(hmode ? th + 2 : th), (unsigned)cp.stride, esz);
+                         (unsigned long long)set.H[i], bk, (unsigned)(halo ? tw + 2 : tw), (unsigned)(halo ? th + 2 : th), (unsigned)cp.stride, esz);
         if (rc) return rc;
     }
     // bulk (TMA) epilogue whenever the output rows are 16-byte aligned (fp32: Cout % 4 == 0; fp16: Cout % 8 == 0, required)
@@ -1748,24 +1418,25 @@ int rf_conv2d_tc(const ImgSet& set, const ConvParams& cp, const void* w_tc, cuda
     p.R = cp.R; p.S = cp.S; p.pad = cp.pad; p.stride = cp.stride; p.Cin = cp.Cin; p.Cout = cp.Cout; p.relu = cp.relu; p.round_out = cp.round_out;
     p.bias = cp.bias; p.residual = cp.residual; p.y = cp.y;
     const int nt = (cp.Cout + BN - 1) / BN;
-    p.raster_n = (raster_mode() && tiles <= 65535) ? 1 : 0;
+    // channel tiles fastest for the tap-streaming kernels: the CTAs of one pixel tile run together (A once from HBM, whole
+    // output rows; +2 % per pair); the grid's y dimension holds at most 65535 pixel tiles
+    p.raster_n = tiles <= 65535 ? 1 : 0;
     const bool deep = cp.K >= 512;                                   // >= 16 K-steps of 32 fp32 channels (8 of 64 fp16)
-    if (f16 && out32) return BN == 128 ? launch_halo<128, true, true>(p, tiles, nt, hmode, st) : launch_halo<64, true, true>(p, tiles, nt, hmode, st);
+    // the weights-resident persistent kernel for 64 -> 64 3x3 convs (a 3-slot / direct-store variant measured no faster:
+    // 332 vs 320 us per pair)
+    const bool resb = halo && cp.Cin == 64 && cp.Cout == 64;
+    if (f16 && out32) return BN == 128 ? launch_halo<128, true, true>(p, tiles, nt, st) : launch_halo<64, true, true>(p, tiles, nt, st);
     if (f16) {
-        if (hmode && resb_mode() && cp.Cin == 64 && cp.Cout == 64) return launch_resb<true>(p, tiles, st);
-        if (hmode) return BN == 128 ? launch_halo<128, true>(p, tiles, nt, hmode, st) : launch_halo<64, true>(p, tiles, nt, hmode, st);
-        const int pm = pipe_mode();
-        if (pm == 1 || (pm == 2 && cp.K >= 4 * TC_BK_F16 && (long long)tiles * nt >= 2ll * num_sms()))
+        if (resb) return launch_resb<true>(p, tiles, st);
+        if (halo) return BN == 128 ? launch_halo<128, true>(p, tiles, nt, st) : launch_halo<64, true>(p, tiles, nt, st);
+        // the pipelined persistent kernel where it measured faster: >= 4 K blocks and >= 2 tiles per SM
+        if (cp.K >= 4 * TC_BK_F16 && (long long)tiles * nt >= 2ll * num_sms())
             return BN == 128 ? launch_pipe<128>(p, tiles, nt, st) : launch_pipe<64>(p, tiles, nt, st);
         if (BN == 128) return deep ? launch_tc<128, MODE_CONV, true, true>(p, tiles, nt, st) : launch_tc<128, MODE_CONV, false, true>(p, tiles, nt, st);
         return deep ? launch_tc<64, MODE_CONV, true, true>(p, tiles, nt, st) : launch_tc<64, MODE_CONV, false, true>(p, tiles, nt, st);
     }
-    if (hmode && resb_mode() && p.tma_epi && cp.Cin == 64 && cp.Cout == 64) return launch_resb<false>(p, tiles, st);
-    if (persist_mode() && p.tma_epi) {
-        if (hmode) return BN == 128 ? launch_persist<128, true>(p, tiles, nt, st) : launch_persist<64, true>(p, tiles, nt, st);
-        return BN == 128 ? launch_persist<128, false>(p, tiles, nt, st) : launch_persist<64, false>(p, tiles, nt, st);
-    }
-    if (hmode) return BN == 128 ? launch_halo<128>(p, tiles, nt, hmode, st) : launch_halo<64>(p, tiles, nt, hmode, st);
+    if (resb && p.tma_epi) return launch_resb<false>(p, tiles, st);
+    if (halo) return BN == 128 ? launch_halo<128>(p, tiles, nt, st) : launch_halo<64>(p, tiles, nt, st);
     if (BN == 128) return deep ? launch_tc<128, MODE_CONV, true>(p, tiles, nt, st) : launch_tc<128, MODE_CONV, false>(p, tiles, nt, st);
     return deep ? launch_tc<64, MODE_CONV, true>(p, tiles, nt, st) : launch_tc<64, MODE_CONV, false>(p, tiles, nt, st);
 }
@@ -1808,15 +1479,6 @@ int rf_stem7_f16_impl(const float* x, int nimg, const int* hw_host, const void* 
 
 size_t rf_corr_tc_workspace(int NA, int NB, int C) { return 2ull * ((size_t)NA + NB) * C * sizeof(float) + 1024; }
 
-// RF_CORR_V2 (read per call): 1 (default) = precision 2 runs the persistent correlation kernel with the fused split /
-// key-zeroing launch in front and the fused flag + compaction kernel behind (3 launches); 0 = the one-tile-per-CTA
-// kernel with separate memset / split / split / flag / compact launches (6).  Identical outputs.
-constexpr int RF_CORR_V2_DEFAULT = 1;      // measured on B200: 178 -> 112 us per call at config 2 (profiles/README.md)
-int rf_corr_v2_mode() {
-    const char* e = getenv("RF_CORR_V2");
-    return e ? atoi(e) : RF_CORR_V2_DEFAULT;
-}
-
 static int launch_corr_pipe(const TcParams& p, int tiles_m, int tiles_n, cudaStream_t st) {
     using Cfg = CorrPipeCfg;
     static bool attr[64] = {false};
@@ -1827,26 +1489,20 @@ static int launch_corr_pipe(const TcParams& p, int tiles_m, int tiles_n, cudaStr
     }
     const long long total = (long long)tiles_m * tiles_n;
     const int grid = total < num_sms() ? (int)total : num_sms();
-    static int mma3 = -1;
-    if (mma3 < 0) { const char* e = getenv("RF_CORR_MMA3"); mma3 = (e && atoi(e) != 0) ? 1 : 0; }
-    TcParams q = p;
-    q.stages = mma3 ? 3 : 0;              // this kernel's ring depth is fixed; the field selects the MMA sequence
-    tc_corr_pipe_kernel<<<grid, TC_THREADS, Cfg::SMEM_BYTES, st>>>(q, tiles_m, tiles_n);
+    tc_corr_pipe_kernel<<<grid, TC_THREADS, Cfg::SMEM_BYTES, st>>>(p, tiles_m, tiles_n);
     RF_LAUNCHED();
     return 0;
 }
 
-// v2 (precision 2 only): the caller has NOT zeroed rowbest / colbest (contiguous, NA + NB keys): the split launch does it
-// presplit (precision 2, v2 only; nullable): {A hi, A lo, B hi, B lo} fp16 planes written by the producer of the features
-// (rf_l2norm_split_nhwc): no split launch; the caller has zeroed the keys.
-// tail (nullable; v2 only): {idx1, idx2, count, done_counter} - the persistent kernel's last CTA also runs the mutual test and
-// the compaction (NA <= 49152: the row table lives in the idle operand ring); done_counter is zeroed by the caller.
+// precision 1: 3xTF32 one-tile-per-CTA kernel; the caller has zeroed rowbest / colbest.
+// precision 2: the persistent fp16-split kernel.  presplit (nullable): {A hi, A lo, B hi, B lo} fp16 planes written by the
+// producer of the features (rf_l2norm_split_nhwc): no split launch, the caller has zeroed the keys.  Without presplit the
+// split launch zeroes rowbest / colbest (contiguous, NA + NB keys).
 int rf_corr_argmax_tc(const float* featA, int NA, const float* featB, int NB, int C,
-                      unsigned long long* rowbest, unsigned long long* colbest, void* ws, cudaStream_t st, int precision, bool v2,
-                      const void* const* presplit, void* const* tail) {
+                      unsigned long long* rowbest, unsigned long long* colbest, void* ws, cudaStream_t st, int precision,
+                      const void* const* presplit) {
     const bool f16 = precision == 2;
-    RF_REQUIRE(presplit == nullptr || (v2 && f16), "rf_corr_mutual_nn: pre-split operands go with the persistent fp16-split kernel");
-    RF_REQUIRE(!v2 || f16, "rf_corr_mutual_nn: the persistent correlation kernel is the fp16-split one (precision 2)");
+    RF_REQUIRE(presplit == nullptr || f16, "rf_corr_mutual_nn: pre-split operands go with the persistent fp16-split kernel");
     RF_REQUIRE((C % (f16 ? TC_BK_F16 : TC_BK)) == 0, "rf_corr_mutual_nn: precision 1 needs C % 32 == 0, precision 2 C % 64 == 0");
     uintptr_t base = (reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255;
     const size_t esz = f16 ? 2 : 4;
@@ -1861,16 +1517,11 @@ int rf_corr_argmax_tc(const float* featA, int NA, const float* featB, int NB, in
         Bhi = const_cast<char*>(static_cast<const char*>(presplit[2]));
         Blo = const_cast<char*>(static_cast<const char*>(presplit[3]));
         for (int i = 0; i < 4; ++i) RF_REQUIRE(presplit[i] != nullptr && ((uintptr_t)presplit[i] % 16) == 0, "rf_corr_mutual_nn_presplit: planes must be 16-byte aligned");
-    } else if (v2) {
+    } else if (f16) {
         RF_REQUIRE(colbest == rowbest + NA, "rf_corr_mutual_nn: arg-max keys must be contiguous");
         const long long nkeys = (long long)NA + NB, n = na4 + nb4 > nkeys ? na4 + nb4 : nkeys;
         split_f16_all_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const float4*)featA, (const float4*)featB, (uint2*)Ahi, (uint2*)Alo,
                                                                             (uint2*)Bhi, (uint2*)Blo, na4, nb4, rowbest, nkeys);
-        RF_LAUNCHED();
-    } else if (f16) {
-        split_f16_kernel<<<(unsigned)((na4 + 255) / 256), 256, 0, st>>>((const float4*)featA, (uint2*)Ahi, (uint2*)Alo, na4);
-        RF_LAUNCHED();
-        split_f16_kernel<<<(unsigned)((nb4 + 255) / 256), 256, 0, st>>>((const float4*)featB, (uint2*)Bhi, (uint2*)Blo, nb4);
         RF_LAUNCHED();
     } else {
         split_tf32_kernel<<<(unsigned)((na4 + 255) / 256), 256, 0, st>>>((const float4*)featA, (float4*)Ahi, (float4*)Alo, na4);
@@ -1878,9 +1529,7 @@ int rf_corr_argmax_tc(const float* featA, int NA, const float* featB, int NB, in
         split_tf32_kernel<<<(unsigned)((nb4 + 255) / 256), 256, 0, st>>>((const float4*)featB, (float4*)Bhi, (float4*)Blo, nb4);
         RF_LAUNCHED();
     }
-    // optional 256-wide score tiles (RF_CORR_BN=256, 3xTF32 only): the featA slab (hi + lo) is fetched once per 256 columns
-    const bool wide = !f16 && NB > 128 && corr_tile_n() == 256;
-    const int BN = wide ? 256 : 128;
+    const int BN = 128;
     const unsigned bk = f16 ? TC_BK_F16 : TC_BK, es = (unsigned)esz;
     TcParams p;
     memset(&p, 0, sizeof(p));
@@ -1897,15 +1546,6 @@ int rf_corr_argmax_tc(const float* featA, int NA, const float* featB, int NB, in
     if (rc) return rc;
     p.R = 1; p.S = 1; p.pad = 0; p.stride = 1; p.Cin = C; p.Cout = NB;
     p.rowbest = rowbest; p.colbest = colbest; p.NA = NA; p.NB = NB;
-    if (tail != nullptr) {
-        RF_REQUIRE(v2 && (size_t)NA * sizeof(int) <= (size_t)CorrPipeCfg::OFF_T, "rf_corr_mutual_nn: fused compaction needs the persistent kernel and NA <= 49152");
-        p.tail_idx1 = static_cast<long long*>(tail[0]);
-        p.tail_idx2 = static_cast<long long*>(tail[1]);
-        p.tail_count = static_cast<int*>(tail[2]);
-        p.done_counter = static_cast<unsigned int*>(tail[3]);
-    }
-    if (v2) return launch_corr_pipe(p, p.tiles_x[0], (NB + 127) / 128, st);
-    if (f16) return launch_tc<128, MODE_CORR, false, true>(p, p.tiles_x[0], (NB + 127) / 128, st);
-    if (wide) return launch_tc<256, MODE_CORR, false>(p, p.tiles_x[0], (NB + 255) / 256, st);
-    return launch_tc<128, MODE_CORR, false>(p, p.tiles_x[0], (NB + 127) / 128, st);
+    if (f16) return launch_corr_pipe(p, p.tiles_x[0], (NB + BN - 1) / BN, st);
+    return launch_tc<BN, MODE_CORR, false>(p, p.tiles_x[0], (NB + BN - 1) / BN, st);
 }

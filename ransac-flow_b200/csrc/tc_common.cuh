@@ -147,35 +147,10 @@ __device__ __forceinline__ void umma_3xtf32_x4(uint32_t tmem_d, uint64_t ahi, ui
         "@e tcgen05.mma.cta_group::1.kind::tf32 [%0], ah, bh, %5, t;\n\t}"
         ::"r"(tmem_d), "l"(ahi), "l"(alo), "l"(bhi), "l"(blo), "r"(idesc), "r"(acc_first) : "memory");
 }
-// fp16 split (correlation precision 2): x = hi + lo * 2^-11 with hi = fp16(x), lo = fp16((x - hi) * 2^11).  Per K = 16 step
-// lo*hi and hi*lo accumulate into `tmem_x` (scaled by 2^11), hi*hi into `tmem_d`; the epilogue adds tmem_x * 2^-11.  Same
-// 22 significand bits as 3xTF32 at half the MMAs per channel (K = 16 per instruction instead of 8).
-__device__ __forceinline__ void umma_f16split_x4(uint32_t tmem_d, uint32_t tmem_x, uint64_t ahi, uint64_t alo, uint64_t bhi, uint64_t blo,
-                                                 uint32_t idesc, uint32_t acc_first) {
-    asm volatile(
-        "{\n\t.reg .pred e, p, t;\n\t.reg .b64 ah, al, bh, bl;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "setp.ne.b32 p, %7, 0;\n\t"
-        "setp.eq.u32 t, 0, 0;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], %3, %4, %6, p;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], %2, %5, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%0], %2, %4, %6, p;\n\t"
-        "add.u64 ah, %2, 2;\n\tadd.u64 al, %3, 2;\n\tadd.u64 bh, %4, 2;\n\tadd.u64 bl, %5, 2;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], al, bh, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], ah, bl, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%0], ah, bh, %6, t;\n\t"
-        "add.u64 ah, %2, 4;\n\tadd.u64 al, %3, 4;\n\tadd.u64 bh, %4, 4;\n\tadd.u64 bl, %5, 4;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], al, bh, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], ah, bl, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%0], ah, bh, %6, t;\n\t"
-        "add.u64 ah, %2, 6;\n\tadd.u64 al, %3, 6;\n\tadd.u64 bh, %4, 6;\n\tadd.u64 bl, %5, 6;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], al, bh, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%1], ah, bl, %6, t;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%0], ah, bh, %6, t;\n\t}"
-        ::"r"(tmem_d), "r"(tmem_x), "l"(ahi), "l"(alo), "l"(bhi), "l"(blo), "r"(idesc), "r"(acc_first) : "memory");
-}
-// The same products with TWO MMAs per K = 16 step instead of three, for operand tiles whose hi and lo B planes are adjacent in
-// shared memory ([N rows hi][N rows lo], N * 128 bytes each) and whose main and cross accumulators are adjacent in TMEM
+// fp16 split: x = hi + lo * 2^-11 with hi = fp16(x), lo = fp16((x - hi) * 2^11).  Per K = 16 step hi*hi accumulates into the
+// main accumulator, lo*hi and hi*lo into the cross one (scaled by 2^11); the epilogue adds cross * 2^-11.  Same 22 significand
+// bits as 3xTF32 at half the MMAs per channel.  The three products take TWO MMAs: the hi and lo B planes are adjacent in
+// shared memory ([N rows hi][N rows lo], N * 128 bytes each) and the main and cross accumulators are adjacent in TMEM
 // ([tmem_d, tmem_d + N) main, [tmem_d + N, tmem_d + 2N) cross):
 //   A hi x [B hi | B lo]  as ONE N' = 2N instruction  -> main += hi*hi, cross += hi*lo
 //   A lo x  B hi                                      -> cross += lo*hi

@@ -8,7 +8,6 @@ restated on the library's kernels (no file IO, no metrics: those stay in the dri
   KITTI        : evaluation/evalKITTI/evaluation.py:49-100,216-344 (two-level flow, small connected components),
                  evaluation/evalKITTI/getResults.py:95-141 (two-level recomposition)
 """
-import os
 
 import numpy as np
 import torch
@@ -23,15 +22,6 @@ def base_grid(h, w, device="cuda"):
     gy = torch.linspace(-1, 1, steps=h, device=device).view(1, -1, 1, 1).expand(1, h, w, 1)
     gx = torch.linspace(-1, 1, steps=w, device=device).view(1, 1, -1, 1).expand(1, h, w, 1)
     return torch.cat((gx, gy), dim=3).contiguous()
-
-
-CORR_NEIGH_PAIR_DEFAULT = "1"
-
-
-def _corr_neigh_pair():
-    """RF_CORR_NEIGH_PAIR=1 (default): PredFlowMask computes corr12 and corr21 with one launch (``ops.corr_neigh_pair``) instead of two
-    launches and a concatenation.  Bit-identical volumes (tests/test_gpu_ops.py)."""
-    return os.environ.get("RF_CORR_NEIGH_PAIR", CORR_NEIGH_PAIR_DEFAULT) != "0"
 
 
 def fine_features(netFeatCoarse, img):
@@ -62,16 +52,12 @@ def PredFlowMask_device(IsTensor, featt, flowCoarse, size, network, with_match21
         tc = model.fine_engine()            # 0 plain fp32, 1 TF32-rounded, 2 fp16, 4 split planes: the operand type of the heads
         if tc == ops.ENGINE_SPLIT:              # one launch: corr12 standalone + the two-image [corr12 ; corr21] tensor, split planes
             corr12, both = ops.corr_neigh_pair_split(ft, fs, k, ld)
-        elif _corr_neigh_pair():                # both volumes from one launch, already laid out as the two-image batch
+        else:                                   # both volumes from one launch, already laid out as the two-image batch
             corr12, corr21, both = ops.corr_neigh_pair(ft, fs, k, ld, tc)
-        else:
-            corr12 = ops.corr_neigh(ft, fs, k, ld, tc)
-            corr21 = ops.corr_neigh(fs, ft, k, ld, tc)
-            both = Ragged(torch.cat([corr12.data, corr21.data], dim=0), corr12.hw + corr21.hw)
         # the two heads are independent: the flow head (one image: 152 tiles in its widest layer, i.e. one full wave + 4 tiles on 148
         # SMs) runs on the side stream and fills the tails of the matchability head's kernels (two images) and vice versa
         main, side = torch.cuda.current_stream(), _side_stream()
-        if _HEADS_TWO_STREAMS and side != main:
+        if side != main:
             side.wait_stream(main)
             with torch.cuda.stream(side):
                 flowDown8 = network["netFlowCoarse"].forward_ragged(corr12)
@@ -102,8 +88,6 @@ def PredFlowMask(IsTensor, featt, flowCoarse, grid, network, with_match21=False,
 
 _pinned = {}
 _side = {}
-_HEADS_TWO_STREAMS = os.environ.get("RF_HEADS_TWO_STREAMS", "1") != "0"
-_FE_BATCH = os.environ.get("RF_FE_BATCH", "1") != "0"          # sync-free paths: FeatureExtractor on [warped source, target] as one batch
 
 
 def _side_stream():
@@ -126,29 +110,13 @@ def _to_host(t):
 
 def _single_device(coarseModel, network, Is, It, with_match21, samples=None):
     """Device part of the single-hypothesis path: everything queued on the current stream, nothing read back."""
-    # the target's fine features do not depend on the coarse stage: queue them on a second stream as soon as the resized
-    # target exists, so they fill the SMs that the small late layers of the ResNet trunk, the matching and RANSAC leave idle
-    main = torch.cuda.current_stream()
-    side = _side_stream()
-    box = {}
-    batch_fe = _FE_BATCH
-
-    def start_target_features():
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            box["featt"] = fine_features(network["netFeatCoarse"], coarseModel.ItTensor)
-    coarseModel.setPair(Is, It, after_preproc=None if batch_fe else start_target_features)
+    coarseModel.setPair(Is, It)
     Itw, Ith = coarseModel.target_size
     Hd, nb, mask, status, cnt = coarseModel.getCoarse_device(None, samples)
     flowCoarse = ops.warp_grid(Hd.view(1, 3, 3), Ith, Itw)
-    if batch_fe:        # target and warped source through the FeatureExtractor as one two-image batch (bit-identical features)
-        flow12, match, f8, mboth = PredFlowMask_device(coarseModel.IsTensor, None, flowCoarse, (Ith, Itw), network, with_match21,
-                                                       ItTensor=coarseModel.ItTensor)
-    else:
-        main.wait_stream(side)
-        featt = box["featt"]
-        featt.data.record_stream(main)
-        flow12, match, f8, mboth = PredFlowMask_device(coarseModel.IsTensor, featt, flowCoarse, (Ith, Itw), network, with_match21)
+    # target and warped source through the FeatureExtractor as one two-image batch (bit-identical features)
+    flow12, match, f8, mboth = PredFlowMask_device(coarseModel.IsTensor, None, flowCoarse, (Ith, Itw), network, with_match21,
+                                                   ItTensor=coarseModel.ItTensor)
     packed = torch.cat([status.float(), cnt.float(), nb.float(), Hd, match.reshape(-1), f8.reshape(-1), mboth.reshape(-1)])
     return packed, flow12, (Ith, Itw), tuple(f8.shape)
 
@@ -313,16 +281,8 @@ def _multi_device(coarseModel, network, Is, It, maxCoarse, maskRegionTh, with_ma
     would have had; dead ones are wasted work (none when every hypothesis is accepted, the common case at maxCoarse = 10).
     One packed result tensor: per hypothesis [alive, status, nbMatch, nbInlier, H(9), flowDown8, matchDown8] - the tensors
     the drivers save (evaluation.py:244-260); the full-resolution maps stay on the device and are not returned."""
-    main = torch.cuda.current_stream()
-    side = _side_stream()
     box = {}
-
-    def start_target_features():
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            box["featt"] = fine_features(network["netFeatCoarse"], coarseModel.ItTensor)
-    batch_fe = _FE_BATCH
-    coarseModel.setPair(Is, It, after_preproc=None if batch_fe else start_target_features)
+    coarseModel.setPair(Is, It)
     Itw, Ith = coarseModel.target_size
     dev = coarseModel.ItTensor.device
     Mask = torch.zeros((Ith, Itw), device=dev)
@@ -332,10 +292,6 @@ def _multi_device(coarseModel, network, Is, It, maxCoarse, maskRegionTh, with_ma
         fgMask = (Mask > 0.5).float()                                    # It_bg = 1 everywhere: (Mask + (1 - It_bg)) > 0.5
         Hd, nb, mask, status, cnt = coarseModel.getCoarse_device(fgMask if k > 0 else None, None if samples is None else samples[k])
         flowCoarse = ops.warp_grid(Hd.view(1, 3, 3), Ith, Itw)
-        if featt is None and not batch_fe:
-            main.wait_stream(side)
-            featt = box["featt"]
-            featt.data.record_stream(main)
         flow12, match, f8, mboth = PredFlowMask_device(coarseModel.IsTensor, featt, flowCoarse, (Ith, Itw), network, with_match21,
                                                        ItTensor=coarseModel.ItTensor, feat_box=box)
         if featt is None:

@@ -1,5 +1,5 @@
 """Stand-alone launches of the hot kernels at config-2 shapes (for ncu captures and CUDA-event timing).
-Usage: python scripts/kernel_bench.py {corr|corr2|corr2v|ransac|conv|c64} [reps]"""
+Usage: python scripts/kernel_bench.py {corr|corr2|ransac|conv|c64} [reps]"""
 import os
 import sys
 
@@ -39,22 +39,14 @@ if which == "corr":
     for prec in (2, 1, 0):
         m, mn = timed(lambda: rf.ops.corr_mutual_nn(A, B, prec))
         print("corr_mutual_nn precision=%d: mean %.1f us, min %.1f us -> %.1f TFLOP/s algorithmic" % (prec, m * 1e3, mn * 1e3, 32.108544 / m))
-elif which in ("corr2", "corr2v"):
-    # precision 2 only: the one-tile-per-CTA kernel sequence (RF_CORR_V2=0) against the persistent one (RF_CORR_V2=1);
-    # corr2v runs only the persistent one (for ncu captures)
+elif which == "corr2":                  # precision 2 only
     g = torch.Generator(device="cpu").manual_seed(0)
     A = torch.nn.functional.normalize(torch.rand(13065, 1024, generator=g), dim=1).to(dev)
     B = torch.nn.functional.normalize(torch.rand(1200, 1024, generator=g), dim=1).to(dev)
-    res = {}
-    for v2 in (("1",) if which == "corr2v" else ("0", "1", "0", "1")):
-        os.environ["RF_CORR_V2"] = v2
-        m, mn = timed(lambda: rf.ops.corr_mutual_nn(A, B, 2))
-        i1, i2, n = rf.ops.corr_mutual_nn(A, B, 2)
-        res[v2] = (i1[:int(n)].cpu(), i2[:int(n)].cpu())
-        print("corr_mutual_nn precision=2 RF_CORR_V2=%s (%d launches): mean %.1f us, min %.1f us -> %.1f TFLOP/s algorithmic, %d pairs"
-              % (v2, rf._lib.lib.rf_corr_mutual_nn_launches(2), m * 1e3, mn * 1e3, 32.108544 / m, int(n)))
-    if len(res) == 2:
-        print("identical pair lists:", bool(torch.equal(res["0"][0], res["1"][0]) and torch.equal(res["0"][1], res["1"][1])))
+    m, mn = timed(lambda: rf.ops.corr_mutual_nn(A, B, 2))
+    i1, i2, n = rf.ops.corr_mutual_nn(A, B, 2)
+    print("corr_mutual_nn precision=2 (%d launches): mean %.1f us, min %.1f us -> %.1f TFLOP/s algorithmic, %d pairs"
+          % (rf._lib.lib.rf_corr_mutual_nn_launches(2), m * 1e3, mn * 1e3, 32.108544 / m, int(n)))
 elif which == "ransac":
     m1, m2, _ = synth.make_matches(1, 636, 0.6)
     t1, t2 = torch.from_numpy(m1).to(dev), torch.from_numpy(m2).to(dev)
@@ -70,7 +62,7 @@ elif which == "c64":
     fc = rf.model.FoldedConv(w, None, 1)
     m, mn = timed(lambda: fc(x, relu=True, engine=1))
     fl = 2.0 * P * 64 * 64 * 9 / 1e9
-    print("conv3x3 64->64 on %d px (RF_TC_RESB=%s): mean %.1f us -> %.1f TFLOP/s" % (P, os.environ.get("RF_TC_RESB", "0"), m * 1e3, fl / m))
+    print("conv3x3 64->64 on %d px: mean %.1f us -> %.1f TFLOP/s" % (P, m * 1e3, fl / m))
 else:
     sizes = [(60, 80), (50, 66), (40, 53), (30, 40), (25, 33), (20, 26), (15, 20), (30, 40)]      # layer3 grids of config 2
     P = sum(h * w for h, w in sizes)

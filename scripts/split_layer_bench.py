@@ -1,7 +1,6 @@
 """CUDA-event timing of the ResNet-50 trunk's layer shapes on the split engine (rf_conv2d_nhwc engine 4) at config-2 sizes:
 the 8 images of one pair (7 source scales + target).  One line per distinct layer shape, L2 flushed between launches, and the
-trunk total weighted by how often each shape occurs.  The library reads its RF_SPLIT_* switches once per process, so variants
-are compared by running this script once per environment.
+trunk total weighted by how often each shape occurs.
 Usage: python scripts/split_layer_bench.py [reps]"""
 import os
 import sys
@@ -50,7 +49,6 @@ def split_ragged(sizes, c, g):
 def main():
     g = torch.Generator(device=dev).manual_seed(0)
     total = 0.0
-    print("RF_SPLIT_EPW=%s RF_SPLIT_BN=%s RF_SPLIT_RES2=%s" % tuple(os.environ.get(k, "-") for k in ("RF_SPLIT_EPW", "RF_SPLIT_BN", "RF_SPLIT_RES2")))
     for name, sizes, cin, cout, k, stride, res, count in LAYERS:
         x = split_ragged(sizes, cin, g)
         ws = rf.ops.to_split(torch.randn(cout, k * k * cin, generator=g, device=dev) / np.sqrt(k * k * cin))

@@ -35,16 +35,11 @@ def test_workspace_queries_are_host_only(rf):
     assert rf._lib.lib.rf_corr_mutual_nn_workspace(13065, 1200, 1024, 0) >= (13065 + 1200) * 8
 
 
-def test_corr_kernel_sequence_query_follows_the_switch(rf, monkeypatch):
-    """rf_corr_mutual_nn_launches is host-only: 4 launches for the fp32 kernel, 6 for the tensor-core kernels with separate
-    helpers, 3 for precision 2 on the persistent kernel sequence (RF_CORR_V2, read per call)."""
+def test_corr_kernel_sequence_query(rf):
+    """rf_corr_mutual_nn_launches is host-only: 4 launches for the fp32 kernel, 6 for the 3xTF32 kernel with separate
+    helpers, 3 for precision 2 (fused split / zeroing, persistent kernel, fused mutual test + compaction)."""
     L = rf._lib.lib
-    monkeypatch.setenv("RF_CORR_V2", "0")
-    assert (L.rf_corr_mutual_nn_launches(0), L.rf_corr_mutual_nn_launches(1), L.rf_corr_mutual_nn_launches(2)) == (4, 6, 6)
-    monkeypatch.setenv("RF_CORR_V2", "1")
     assert (L.rf_corr_mutual_nn_launches(0), L.rf_corr_mutual_nn_launches(1), L.rf_corr_mutual_nn_launches(2)) == (4, 6, 3)
-    monkeypatch.delenv("RF_CORR_V2")
-    assert L.rf_corr_mutual_nn_launches(2) in (3, 6)
 
 
 def test_lanczos_coefficients_match_pil(rf):

@@ -76,16 +76,16 @@ def test_conv2d_f16(rf, cin, cout, k, sizes, relu, res, stride):
         assert err <= F16_TOL * max(1.0, r.abs().max().item()), (err, r.abs().max().item())
 
 
-@pytest.mark.parametrize("env", [{"RF_TC_PIPE": "1"}, {"RF_TC_PIPE": "0", "RF_TC_RASTER": "0"}, {"RF_TC_PIPE": "0", "RF_TC_RESPF": "1"},
-                                 {"RF_TC_PIPE": "1", "RF_TC_RASTER": "0"}])
+@pytest.mark.parametrize("env", [{}, {"RF_TC_RESPF": "1"}])
 @pytest.mark.parametrize("cin,cout,k,stride,res,sizes", [
     (64, 256, 1, 1, True, [(120, 160), (60, 80), (33, 47)]), (256, 64, 1, 1, False, [(120, 160), (31, 17)]),
     (512, 1024, 1, 2, False, [(60, 80), (30, 44)]), (128, 128, 3, 2, False, [(64, 96), (37, 41)]),
-    (256, 1024, 1, 1, True, [(30, 40), (60, 80), (15, 20)]), (128, 512, 1, 1, True, [(9, 7)])])
+    (256, 1024, 1, 1, True, [(30, 40), (60, 80), (15, 20)]), (128, 512, 1, 1, True, [(9, 7)]),
+    (256, 64, 1, 1, False, [(240, 320)])])                                  # 600 tiles: tc_pipe_kernel<64>
 def test_conv2d_f16_kernel_variants(rf, monkeypatch, env, cin, cout, k, stride, res, sizes):
-    """The same fp16 convolutions through every tap-streaming kernel variant (the switches are read per call): the
-    pipelined persistent kernel (two epilogue groups, producer-issued residual prefetch), pixel-tile-fastest raster,
-    and the residual-prefetching one-tile kernel.  All must agree with the fp32 reference."""
+    """fp16 tap-streaming convolutions on both sides of the kernel selection: the pipelined persistent kernel (two
+    epilogue groups, producer-issued residual prefetch; >= 4 K blocks and >= 2 tiles per SM) and the one-tile kernel,
+    also with its residual prefetch (RF_TC_RESPF, read per call).  All must agree with the fp32 reference."""
     for kk, v in env.items():
         monkeypatch.setenv(kk, v)
     g = torch.Generator().manual_seed(cin + cout + k + stride)
@@ -175,11 +175,11 @@ def test_corr_kitti_shape_both_engines_agree(rf):
 
 @pytest.mark.parametrize("C,NA,NB,seed", [(1024, 13065, 1200, 0), (1024, 2107, 300, 1), (64, 129, 127, 2), (256, 1, 1, 4),
                                            (1024, 300, 1200, 5), (128, 5000, 130, 6), (64, 128, 128, 7), (192, 40000, 257, 8)])
-def test_corr_persistent_kernel_identical_to_one_tile_kernel(rf, monkeypatch, C, NA, NB, seed):
-    """Precision 2 has two kernel sequences (RF_CORR_V2, read per call): the persistent correlation kernel (two TMEM
-    accumulator pairs, arg-max epilogue overlapped with the next tile's MMAs, fused split / zeroing and fused mutual test +
-    compaction) must return exactly the pairs of the one-tile-per-CTA kernel - same MMAs, same (score, smallest index)
-    order - and both agree with the fp32 oracle up to arg-max ties below fp32 accumulation noise."""
+def test_corr_persistent_kernel_sequence(rf, C, NA, NB, seed):
+    """Precision 2 runs three launches: fused split / key zeroing, the persistent correlation kernel (two TMEM accumulator
+    pairs, arg-max epilogue overlapped with the next tile's MMAs), fused mutual test + compaction.  Its pairs come in row
+    order and agree with the fp32 oracle and with the library's exact-fp32 kernel up to arg-max ties below fp32
+    accumulation noise."""
     rs = np.random.RandomState(seed)
     A = np.abs(rs.randn(C, NA)).astype(np.float32)
     B = np.abs(rs.randn(C, NB)).astype(np.float32)
@@ -190,27 +190,26 @@ def test_corr_persistent_kernel_identical_to_one_tile_kernel(rf, monkeypatch, C,
     if NB > 2:
         B[:, 1] = 0                              # masked target cell: never matches
     fa, fb = torch.from_numpy(A.T.copy()).cuda(), torch.from_numpy(B.T.copy()).cuda()
-    got = {}
-    for v2 in ("0", "1"):
-        monkeypatch.setenv("RF_CORR_V2", v2)
-        assert rf._lib.lib.rf_corr_mutual_nn_launches(2) == (3 if v2 == "1" else 6)
-        for rep in range(2):                     # twice: the workspace keys must be re-zeroed by the call itself
-            i1, i2, cnt = rf.ops.corr_mutual_nn(fa, fb, 2)
-        k = int(cnt.item())
-        got[v2] = (i1[:k].cpu().numpy(), i2[:k].cpu().numpy())
-    assert np.array_equal(got["0"][0], got["1"][0]) and np.array_equal(got["0"][1], got["1"][1])
-    assert np.all(np.diff(got["1"][0]) > 0)
-    if NA * NB <= 13065 * 1200:
-        o1, o2, score = OO.mutualMatching(A, B, return_score=True)
-        check_same(got["1"][0], got["1"][1], o1, o2, score)
+    assert rf._lib.lib.rf_corr_mutual_nn_launches(2) == 3
+    for rep in range(2):                         # twice: the workspace keys must be re-zeroed by the call itself
+        i1, i2, cnt = rf.ops.corr_mutual_nn(fa, fb, 2)
+    k = int(cnt.item())
+    got = (i1[:k].cpu().numpy(), i2[:k].cpu().numpy())
+    assert np.all(np.diff(got[0]) > 0)
+    o1, o2, score = OO.mutualMatching(A, B, return_score=True)
+    check_same(got[0], got[1], o1, o2, score)
+    j1, j2, n0 = rf.ops.corr_mutual_nn(fa, fb, 0)
+    n0 = int(n0.item())
+    check_same(got[0], got[1], j1[:n0].cpu().numpy(), j2[:n0].cpu().numpy(), score)
 
 
 @pytest.mark.parametrize("C,NA,NB,seed", [(1024, 13065, 1200, 0), (1024, 2107, 300, 1), (64, 129, 127, 2), (256, 1, 1, 4), (1024, 300, 1200, 5),
-                                           (1024, 25747, 8250, 7)])
-def test_corr_presplit_operands_and_column_compaction_identical(rf, monkeypatch, C, NA, NB, seed):
-    """rf_corr_mutual_nn_presplit (operand planes written by rf_l2norm_split_nhwc, key memset, persistent kernel whose last CTA
-    runs the mutual test + compaction) == rf_corr_mutual_nn at precision 2 (split launch + separate compaction): identical
-    index lists, also with the separate column-driven / row-driven compaction kernels (RF_CORR_TAIL, RF_COMPACT_COLS)."""
+                                           (1024, 25747, 8250, 7), (64, 60000, 300, 8)])
+def test_corr_presplit_operands_and_column_compaction_identical(rf, C, NA, NB, seed):
+    """rf_corr_mutual_nn_presplit (operand planes written by rf_l2norm_split_nhwc, key memset, persistent kernel, compaction)
+    == rf_corr_mutual_nn at precision 2 (split launch, persistent kernel, compaction): identical index lists.  The
+    compaction is column-driven while NA row flags fit in shared memory (NA <= 51200) and row-driven beyond; the largest
+    shape takes the row-driven kernel in both calls and is also checked against the fp32 oracle."""
     g = torch.Generator().manual_seed(seed)
     raw = torch.cat([torch.randn(NA + NB, C, generator=g).abs()]).cuda()
     raw[NA:NA + min(NA, NB) // 2] = raw[torch.randperm(NA, generator=g)[:min(NA, NB) // 2].cuda()] + 0.05 * raw[NA:NA + min(NA, NB) // 2]
@@ -220,13 +219,14 @@ def test_corr_presplit_operands_and_column_compaction_identical(rf, monkeypatch,
     rows = rf.ops.from_split(planes)                              # the fp32 values those planes stand for
     ref = rf.ops.corr_mutual_nn(rows[:NA].contiguous(), rows[NA:].contiguous(), 2)
     nref = int(ref[2].item())
-    for tail, cols in (("1", "1"), ("0", "1"), ("0", "0")):        # fused tail in the correlation kernel / column-driven / row-driven kernel
-        monkeypatch.setenv("RF_CORR_TAIL", tail)
-        monkeypatch.setenv("RF_COMPACT_COLS", cols)
-        for _ in range(2):                                        # twice: the ticket counter is re-zeroed per call
-            got = rf.ops.corr_mutual_nn_presplit(planes[0, :NA], planes[1, :NA], planes[0, NA:], planes[1, NA:])
-            n = int(got[2].item())
-            assert n == nref and torch.equal(got[0][:n], ref[0][:n]) and torch.equal(got[1][:n], ref[1][:n]), (tail, cols)
-        again = rf.ops.corr_mutual_nn(rows[:NA].contiguous(), rows[NA:].contiguous(), 2)
-        assert int(again[2].item()) == nref and torch.equal(again[0][:n], ref[0][:n])
+    for _ in range(2):                                            # twice: the keys are re-zeroed per call
+        got = rf.ops.corr_mutual_nn_presplit(planes[0, :NA], planes[1, :NA], planes[0, NA:], planes[1, NA:])
+        n = int(got[2].item())
+        assert n == nref and torch.equal(got[0][:n], ref[0][:n]) and torch.equal(got[1][:n], ref[1][:n])
+    again = rf.ops.corr_mutual_nn(rows[:NA].contiguous(), rows[NA:].contiguous(), 2)
+    assert int(again[2].item()) == nref and torch.equal(again[0][:n], ref[0][:n])
+    if NA * 4 > 200 * 1024:
+        A, B = rows[:NA].T.cpu().numpy().copy(), rows[NA:].T.cpu().numpy().copy()
+        o1, o2, score = OO.mutualMatching(A, B, return_score=True)
+        check_same(got[0][:n].cpu().numpy(), got[1][:n].cpu().numpy(), o1, o2, score)
     assert nref >= 1 and (NB <= 2 or not bool((ref[1][:nref] == 1).any()))
